@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the comms-rs FIR / mixer / FFT hot path on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload fir64] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload fir64] [--impl b200|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input.  The
 default workload is BASELINE.json configs[1]: one 64-tap complex-f32 FIR
@@ -17,6 +17,8 @@ reference cannot be built in this image) on all host cores instead.
 N > 1: one process per GPU (torchrun); each rank owns one overlap-save segment of
 the stream (its halo is the K samples before it), no data-path collective ->
 weak scaling.
+--dump-outputs DIR: the inputs are a seeded counter-based stream, so two builds run with the same arguments can be
+compared output for output (see dump_output).
 """
 from __future__ import annotations
 
@@ -35,6 +37,7 @@ import numpy as np  # noqa: E402
 METRIC = "FIR/FFT Msamples/s"
 UNIT = "Msamples/s"
 SEED = 20260101
+DUMP_BYTES = 64_000_000  # --dump-outputs: all files of one run together, .npy headers included
 
 WORKLOADS = {
     # name: (kind, samples per step per GPU, algorithmic bytes per input sample, description)
@@ -110,9 +113,15 @@ def parse_args():
     ap.add_argument("--no-gather", dest="gather", action="store_false",
                     help="N > 1: skip the ordered gather of the output segments (timed apart from the kernels)")
     ap.add_argument("--pageable", action="store_true", help="also time the host-pointer call with pageable host buffers")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of each measured workload computed to DIR/<workload>.npy "
+                         "(float32 / float64, at most 64 MB in all: larger outputs are sampled at fixed positions)")
     a = ap.parse_args()
     a.warmup = max(a.warmup, 3)
-    a.steps = max(a.steps, 1)
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs is not None and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     if a.also is None:
         a.also = list(ALSO_DEFAULT) if a.workload == "fir64" and a.impl == "b200" else []
     elif a.also.strip().lower() in ("", "none"):
@@ -122,6 +131,7 @@ def parse_args():
         for w in a.also:
             if w not in WORKLOADS:
                 ap.error(f"unknown workload in --also: {w}")
+    a.dump_bytes = DUMP_BYTES // (1 + len([w for w in a.also if w != a.workload]))
     return a
 
 
@@ -540,6 +550,33 @@ class Job:
         return sharding.halo_state(prev, nstate if nstate is not None else k, interp)
 
 
+def sample_rows(rows, max_rows):
+    """Row indices --dump-outputs keeps of an output of `rows` rows: None (all) when they fit, else one row from each
+    of `max_rows` equal strata at an offset drawn from SEED -- the same positions on every run and every build."""
+    if rows <= max_rows:
+        return None
+    stride = rows // max_rows
+    return np.arange(max_rows, dtype=np.int64) * stride + np.random.default_rng(SEED).integers(0, stride, max_rows)
+
+
+def dump_output(job, torch, path, max_bytes):
+    """Writes the array a caller of the timed path receives from its last step: float32 (complex samples and i16 IQ as
+    (re, im) rows) or float64 (the estimators' result), sampled by sample_rows to at most `max_bytes`."""
+    torch.cuda.synchronize()
+    if job.kind == "est":
+        np.save(path, np.array([job.result.value], dtype=np.float64))
+        return
+    y = job.y
+    if y.is_complex():
+        y = torch.view_as_real(y)
+    elif y.dtype == torch.int16:
+        y = y.view(-1, 2)
+    idx = sample_rows(y.shape[0], max((max_bytes - 4096) // (4 * y[0].numel()), 1))  # 4 KB: room for the .npy header
+    if idx is not None:
+        y = y.index_select(0, torch.from_numpy(idx).to(y.device))
+    np.save(path, y.float().cpu().numpy())
+
+
 ALSO_DEFAULT = ["fft1024", "fft4096", "ifft4096", "fft65536", "chain", "pulse4_b4096", "poly8x1024", "fir64_iq16"]
 NVLINK_GBS_PER_DIR = 900.0  # NVLink 5, per GPU and direction (B200_PROFILING.md)
 
@@ -680,6 +717,10 @@ def measure(cb, torch, dist, args, workload, rank, world, local_rank, steps, war
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     total_ms_max = float(t.item())
     clocks = sampler.summary(t_wall0, t_wall1)
+    if args.dump_outputs:  # before the e2e leg, which some workloads run through the same output buffer
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        name = workload if world == 1 else f"{workload}.rank{rank}"
+        dump_output(job, torch, os.path.join(args.dump_outputs, name + ".npy"), args.dump_bytes // world)
 
     # ---- end to end: host buffers, H2D + kernels + D2H inside the timed region
     e2e = None

@@ -1319,3 +1319,44 @@ def test_cpp_host_graph_conformance():
     r = subprocess.run([os.path.join(host, "test_graph")], capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
     assert "host graph tests ok" in r.stdout
+
+
+# ------------------------------------------------------------------ bench.py --dump-outputs
+def test_bench_dump_outputs_are_reproducible_and_are_what_the_path_computed(cb, oracle, tmp_path):
+    """Two runs with the same arguments dump the same bytes, within the size limit, and the dumped rows of the headline
+    FIR are its outputs at the positions bench.sample_rows names (last timed step: the state is the stream's tail)."""
+    import importlib.util
+    import json
+    import os
+    import subprocess
+    import sys
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    spec = importlib.util.spec_from_file_location("_bench", os.path.join(root, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    dumps = []
+    for run in range(2):
+        d = tmp_path / f"run{run}"
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "2", "--warmup", "3", "--no-e2e",
+                            "--no-cpu", "--also", "freqest,fir64_iq16", "--dump-outputs", str(d)],
+                           capture_output=True, text=True, timeout=600, cwd=tmp_path)
+        assert r.returncode == 0, r.stderr[-3000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 2
+        files = sorted(os.listdir(d))
+        assert files == ["fir64.npy", "fir64_iq16.npy", "freqest.npy"]
+        assert sum(os.path.getsize(d / f) for f in files) <= bench.DUMP_BYTES
+        dumps.append({f: np.load(d / f) for f in files})
+    for f, a in dumps[0].items():
+        assert a.dtype in (np.float32, np.float64) and a.tobytes() == dumps[1][f].tobytes(), f
+    assert dumps[0]["freqest.npy"].shape == (1,) and dumps[0]["freqest.npy"].dtype == np.float64
+    n = bench.WORKLOADS["fir64"][1]
+    y = dumps[0]["fir64.npy"]
+    assert y.shape[1] == 2 and 8 * len(y) <= bench.DUMP_BYTES // 3
+    idx = bench.sample_rows(n, len(y))
+    taps = bench.fir_taps("fir64")
+    pick = [j for j in range(0, len(idx), len(idx) // 200) if idx[j] >= 63][:200]
+    want = [oracle.batch_fir(oracle.synth_uniform_c32(bench.SEED, int(idx[j]) - 63, 64), taps, np.zeros(64, np.complex64))[0][-1]
+            for j in pick]
+    got = y[pick, 0] + 1j * y[pick, 1]
+    assert rel_l2(got, want) <= FIR_TOL

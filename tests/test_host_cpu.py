@@ -213,6 +213,27 @@ def test_bench_reference_arm_prints_contract_line():
     assert line["cpu_baseline"]["kind"] == "port" and line["e2e"]["h2d_bytes_per_step"] == 0
 
 
+def test_bench_rejects_arguments_it_would_not_honour(tmp_path):
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path / "d")]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, timeout=120)
+        assert r.returncode == 2 and "error" in r.stderr, (extra, r.stderr[-2000:])
+    assert not (tmp_path / "d").exists()
+
+
+def test_bench_dump_sample_is_fixed_and_covers_the_output():
+    import importlib.util
+
+    spec = importlib.util.spec_from_file_location("_bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    assert bench.sample_rows(1000, 1000) is None
+    for rows, k in ((1 << 28, 1 << 23), (1001, 1000), (13421773, 777)):
+        idx = bench.sample_rows(rows, k)
+        assert len(idx) == k and idx.tobytes() == bench.sample_rows(rows, k).tobytes()
+        stride = rows // k
+        assert np.array_equal(idx // stride, np.arange(k)) and idx[-1] < rows  # one row in each stratum, in order
+
+
 def test_bench_cpu_leg_runs_for_every_workload_kind():
     # the reference arm / cpu_baseline leg of bench.py for one workload of every kind, on a small sample
     import importlib.util
@@ -562,10 +583,13 @@ def test_hot_kernels_keep_their_register_budgets_and_do_not_spill(cb):
     import shutil
     import subprocess
 
-    if shutil.which("cuobjdump") is None:
-        pytest.skip("cuobjdump not on PATH")
+    # the cuobjdump of the toolkit build.py compiles with, which need not be on PATH
+    nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
+    cuobjdump = shutil.which("cuobjdump") or shutil.which("cuobjdump", path=os.path.dirname(nvcc))
+    if cuobjdump is None:
+        pytest.skip("cuobjdump not found on PATH or beside nvcc")
     lib = os.path.join(ROOT, "comms-rs_b200", "libcomms_b200.so")
-    out = subprocess.run(["cuobjdump", "--dump-resource-usage", lib], capture_output=True, text=True, check=True).stdout
+    out = subprocess.run([cuobjdump, "--dump-resource-usage", lib], capture_output=True, text=True, check=True).stdout
     usage = {}
     for m in re.finditer(r"Function (\S+):\s*\n\s*REG:(\d+) STACK:(\d+)", out):
         usage[m.group(1)] = (int(m.group(2)), int(m.group(3)))
