@@ -979,6 +979,7 @@ int cb_fir_create(const float *taps, size_t ntaps, const float *state, size_t ns
             FIR_TRY(cudaMalloc(&h->tc_img, bytes));
             FIR_TRY(cudaMemcpy(h->tc_img, img.data(), bytes, cudaMemcpyHostToDevice));
             h->tc = FirTcPlan{h->tc_img, inv, force_tc ? (size_t)1 : ((size_t)1 << 16)};
+            h->tc.sample_min = fir_taps_pair_sparse(h->taps.data(), h->k_eff, 1);
         } else if (!want_cuda && h->decim == 1 && h->interp > 1 && fir_ptc_supported(h->k_eff, h->interp, h->taps_real)) {
             // polyphase interpolator on the tensor cores (K3-TC); short banks stay on the CUDA-core
             // polyphase kernel unless forced, long banks (> 16 taps per phase) always use it
@@ -989,6 +990,7 @@ int cb_fir_create(const float *taps, size_t ntaps, const float *state, size_t ns
             FIR_TRY(cudaMalloc(&h->tc_img, bytes));
             FIR_TRY(cudaMemcpy(h->tc_img, img.data(), bytes, cudaMemcpyHostToDevice));
             h->tc = FirTcPlan{h->tc_img, inv, force_tc ? (size_t)1 : ((size_t)1 << 16)};
+            h->tc.sample_min = fir_taps_pair_sparse(h->taps.data(), h->k_eff, h->interp);
         }
     }
         const char *path2 = getenv("COMMS_B200_FIR_PATH");
@@ -1372,7 +1374,8 @@ int cb_fir_run_dev_iq16(cb_fir *h, const int16_t *d_in, size_t n_in, float in_sc
     if (rc) return rc;
     if (fir_iq16_fused(h, n_in, d_in, d_out)) {
         FirSeg seg{nullptr, h->hist[h->cur], h->hist[h->cur ^ 1], nullptr, n_in, no, h->hist_len, h->k_eff, h->interp, h->decim};
-        rc = launch_fir_tc_iq16(seg, d_in, in_scale, d_out, out_scale, h->tc.bimg_dev, h->tc.tap_inv_scale, s);
+        h->tc.fix = fir_fix_for(h, n_in, 0);
+        rc = launch_fir_tc_iq16(seg, d_in, in_scale, d_out, out_scale, h->tc, h->taps_dev, s);
         if (rc) return rc;
         h->cur ^= 1;
         return h->last.end(s);
@@ -1441,8 +1444,9 @@ int cb_fir_run_iq16(cb_fir *h, const int16_t *in, size_t n_in, float in_scale, f
             if (rc) return rc;
             int16_t *y16 = reinterpret_cast<int16_t *>(h->pipe.out[l]);
             FirSeg seg{nullptr, hist_in, last ? h->hist[h->cur ^ 1] : nullptr, nullptr, n, n, h->hist_len, h->k_eff, h->interp, h->decim};
-            rc = launch_fir_tc_iq16(seg, reinterpret_cast<const int16_t *>(slot16 + H * IQ), in_scale, y16, out_scale, h->tc.bimg_dev,
-                                    h->tc.tap_inv_scale, s);
+            h->tc.fix = fir_fix_for(h, n, l);
+            rc = launch_fir_tc_iq16(seg, reinterpret_cast<const int16_t *>(slot16 + H * IQ), in_scale, y16, out_scale, h->tc,
+                                    h->taps_dev, s);
             if (rc) return rc;
             rc = h->pipe.d2h(l, hout + out_done * IQ, y16, n * IQ);
             if (rc) return rc;

@@ -417,7 +417,14 @@ __global__ void __launch_bounds__(256) fir_fixup_kernel(const FirFixArgs a)
             long long idx = (long long)m;
             for (unsigned k = p; k < a.ntaps; k += L, --idx) {
                 float2 xs = make_float2(0.f, 0.f);
-                if (idx >= 0) xs = a.x[idx];
+                if (idx >= 0) {
+                    if (a.x16 != nullptr) {
+                        const uint32_t w = a.x16[idx];
+                        xs = make_float2(__fmul_rn(a.in_scale, (float)(int16_t)(w & 0xFFFFu)), __fmul_rn(a.in_scale, (float)(int16_t)(w >> 16)));
+                    } else {
+                        xs = a.x[idx];
+                    }
+                }
                 else if ((long long)a.hist_len + idx >= 0) xs = a.hist_in[(long long)a.hist_len + idx];
                 const float2 h = __ldg(a.taps + k);
                 re = fmaf(h.x, xs.x, re);
@@ -445,6 +452,23 @@ int launch_fir_fixup(const FirFixArgs &a, cudaStream_t stream)
     return CB_OK;
 }
 
+bool fir_taps_pair_sparse(const float2 *taps, uint32_t ntaps, uint32_t interp)
+{
+    const uint32_t L = interp ? interp : 1;
+    for (uint32_t p = 0; p < L; ++p) {
+        bool any = false, even = false, odd = false;  // adjacent non-zero taps of this phase ending at an even / odd offset
+        for (uint32_t q = 0; p + q * L < ntaps; ++q) {
+            const float2 b = taps[p + q * L];
+            if (b.x == 0.f && b.y == 0.f) continue;
+            any = true;
+            const float2 a = q ? taps[p + (q - 1) * L] : make_float2(0.f, 0.f);
+            if (a.x != 0.f || a.y != 0.f) (q & 1 ? odd : even) = true;
+        }
+        if (any && !(even && odd)) return true;  // a phase without non-zero taps only ever outputs zeros
+    }
+    return false;
+}
+
 bool fir_fuses_i16(const FirSeg &seg, bool taps_real, const FirTcPlan *tcplan)
 {
     return tcplan != nullptr && tcplan->bimg_dev != nullptr && seg.n_in >= tcplan->min_samples && seg.interp > 1 &&
@@ -457,9 +481,8 @@ int launch_fir(const FirSeg &seg, const float2 *taps_dev, const float2 *taps_hos
     if (seg.n_in == 0) return CB_OK;
     if (tcplan != nullptr && tcplan->bimg_dev != nullptr && seg.n_in >= tcplan->min_samples) {
         if (seg.interp == 1 && fir_tc_applicable(seg))
-            return launch_fir_tc(seg, tcplan->bimg_dev, tcplan->tap_inv_scale, tcplan->fix, taps_dev, stream);
-        if (seg.interp > 1 && fir_ptc_applicable(seg, taps_real))
-            return launch_fir_ptc(seg, tcplan->bimg_dev, tcplan->tap_inv_scale, taps_real, tcplan->fix, taps_dev, stream);
+            return launch_fir_tc(seg, *tcplan, taps_dev, stream);
+        if (seg.interp > 1 && fir_ptc_applicable(seg, taps_real)) return launch_fir_ptc(seg, *tcplan, taps_real, taps_dev, stream);
     }
     if (seg.interp == 1 && seg.decim == 1) {
         const uint32_t K = seg.ntaps;

@@ -173,7 +173,8 @@ __device__ __forceinline__ uint32_t trunc_i16(float v)
 // per-thread LDG.128 loads straight into registers are best; with the i16 output the write traffic halves, the
 // exposed load latency of the single loader group becomes the limiter, and a TMA warp that keeps a ring of NRAW
 // raw tiles filled ahead of the converters wins (0.436 -> 0.398 ms).  TMA_LOAD = OUT16.
-template <int L, bool CPLX, bool OUT16, int NRAW>
+// SMIN: the quiet test per symbol (taps that may skip one symbol of every pair, FirTcPlan::sample_min)
+template <int L, bool CPLX, bool OUT16, int NRAW, bool SMIN>
 __global__ void __launch_bounds__(OUT16 ? 512 : 288, 1) fir_ptc_kernel(const __grid_constant__ Args a)  // 512: 128-register cap (14 warps)
 {
     constexpr bool TMA_LOAD = OUT16;
@@ -300,7 +301,7 @@ __global__ void __launch_bounds__(OUT16 ? 512 : 288, 1) fir_ptc_kernel(const __g
                 raw[i] = v;
                 const float pm = fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w)));
                 mx = fmaxf(mx, pm);
-                mnu = min(mnu, __float_as_uint(pm) - 1u);
+                mnu = min(mnu, quiet_key<SMIN>(v, pm));
             }
             if (TMA_LOAD) mbar_arrive(&raw_empty[rs]);  // the raw tile is in registers: the TMA warp may refill the stage
 #pragma unroll
@@ -524,12 +525,12 @@ void fir_ptc_build_image(const float2 *taps, uint32_t ntaps, uint32_t L, bool ta
     }
 }
 
-template <int L, bool CPLX, bool OUT16, int NRAW>
+template <int L, bool CPLX, bool OUT16, int NRAW, bool SMIN>
 static int launch_ptc_raw(const ptc::Args &a, cudaStream_t stream)
 {
     using G = ptc::Geo<L, CPLX>;
     const int SMEM = 2 * G::STAGE + (int)a.ks * (CPLX ? 16384 : 8192) + (OUT16 ? NRAW * G::NEL * 8 : 0) + 1024;
-    auto kern = ptc::fir_ptc_kernel<L, CPLX, OUT16, NRAW>;
+    auto kern = ptc::fir_ptc_kernel<L, CPLX, OUT16, NRAW, SMIN>;
     CB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
     const int KT = 16 * (int)a.ks;
     const unsigned long long TS = (unsigned long long)(((G::NEL - KT) / G::RS + 1) * G::RS);
@@ -546,12 +547,13 @@ static int launch_ptc_raw(const ptc::Args &a, cudaStream_t stream)
 
 // two raw stages when they fit in shared memory, else one
 template <int L, bool CPLX, bool OUT16>
-static int launch_ptc_l(const ptc::Args &a, cudaStream_t stream)
+static int launch_ptc_l(const ptc::Args &a, bool smin, cudaStream_t stream)
 {
     using G = ptc::Geo<L, CPLX>;
     const size_t need2 = 2 * (size_t)G::STAGE + (size_t)a.ks * (CPLX ? 16384 : 8192) + 2 * (size_t)G::NEL * 8 + 1024;
-    if (!OUT16 || need2 <= 227 * 1024) return launch_ptc_raw<L, CPLX, OUT16, 2>(a, stream);
-    return launch_ptc_raw<L, CPLX, OUT16, 1>(a, stream);
+    if (!OUT16 || need2 <= 227 * 1024)
+        return smin ? launch_ptc_raw<L, CPLX, OUT16, 2, true>(a, stream) : launch_ptc_raw<L, CPLX, OUT16, 2, false>(a, stream);
+    return smin ? launch_ptc_raw<L, CPLX, OUT16, 1, true>(a, stream) : launch_ptc_raw<L, CPLX, OUT16, 1, false>(a, stream);
 }
 
 bool fir_ptc_applicable(const FirSeg &seg, bool taps_real)
@@ -571,11 +573,11 @@ static unsigned ptc_tile_symbols(uint32_t interp, unsigned ks)
     return (unsigned)(((nel - kt) / rs + 1) * rs);
 }
 
-static int launch_fir_ptc_main(const FirSeg &seg, const ptc::Args &a, bool taps_real, cudaStream_t stream);
+static int launch_fir_ptc_main(const FirSeg &seg, const ptc::Args &a, bool taps_real, bool smin, cudaStream_t stream);
 
-int launch_fir_ptc(const FirSeg &seg, const void *himg_dev, float tap_inv_scale, bool taps_real, FirFix *fix,
-                   const float2 *taps_dev, cudaStream_t stream)
+int launch_fir_ptc(const FirSeg &seg, const FirTcPlan &plan, bool taps_real, const float2 *taps_dev, cudaStream_t stream)
 {
+    FirFix *fix = plan.fix;
     if (seg.n_in == 0) return CB_OK;
     ptc::Args a;
     a.ks = (unsigned)fir_ptc_ksteps(seg.ntaps, seg.interp);
@@ -584,17 +586,17 @@ int launch_fir_ptc(const FirSeg &seg, const void *himg_dev, float tap_inv_scale,
     a.y = seg.y;
     a.hist_in = seg.hist_in;
     a.hist_out = seg.hist_out;
-    a.himg = reinterpret_cast<const uint4 *>(himg_dev);
+    a.himg = reinterpret_cast<const uint4 *>(plan.bimg_dev);
     a.n = seg.n_in;
     a.hist_len = seg.hist_len;
-    a.tap_inv_scale = tap_inv_scale;
+    a.tap_inv_scale = plan.tap_inv_scale;
     a.y16 = reinterpret_cast<int2 *>(seg.y16);
     a.qscale = seg.qscale;
     const unsigned ts = ptc_tile_symbols(seg.interp, a.ks);
     const bool fixup = fix != nullptr && fix->dev != nullptr && taps_dev != nullptr && fix->cap >= ceil_div(seg.n_in, (size_t)ts);
     a.fix_count = fixup ? fix->dev + (fix->calls & 1u) : nullptr;
     a.fix_list = fixup ? fix->dev + 2 : nullptr;
-    const int rc = launch_fir_ptc_main(seg, a, taps_real, stream);
+    const int rc = launch_fir_ptc_main(seg, a, taps_real, plan.sample_min, stream);
     if (rc || !fixup) return rc;
     FirFixArgs f{seg.x, seg.hist_in, taps_dev, seg.y, seg.y16, seg.qscale, seg.n_in, seg.ntaps, seg.interp, ts, seg.hist_len,
                  a.fix_count, fix->dev + ((fix->calls + 1) & 1u), a.fix_list};
@@ -602,18 +604,18 @@ int launch_fir_ptc(const FirSeg &seg, const void *himg_dev, float tap_inv_scale,
     return launch_fir_fixup(f, stream);
 }
 
-static int launch_fir_ptc_main(const FirSeg &seg, const ptc::Args &a, bool taps_real, cudaStream_t stream)
+static int launch_fir_ptc_main(const FirSeg &seg, const ptc::Args &a, bool taps_real, bool smin, cudaStream_t stream)
 {
     if (seg.y16 != nullptr) {
         switch (seg.interp) {
-        case 8: return taps_real ? launch_ptc_l<8, false, true>(a, stream) : launch_ptc_l<8, true, true>(a, stream);
-        case 4: return taps_real ? launch_ptc_l<4, false, true>(a, stream) : launch_ptc_l<4, true, true>(a, stream);
+        case 8: return taps_real ? launch_ptc_l<8, false, true>(a, smin, stream) : launch_ptc_l<8, true, true>(a, smin, stream);
+        case 4: return taps_real ? launch_ptc_l<4, false, true>(a, smin, stream) : launch_ptc_l<4, true, true>(a, smin, stream);
         default: break;
         }
     }
     switch (seg.interp) {
-    case 8: return taps_real ? launch_ptc_l<8, false, false>(a, stream) : launch_ptc_l<8, true, false>(a, stream);
-    case 4: return taps_real ? launch_ptc_l<4, false, false>(a, stream) : launch_ptc_l<4, true, false>(a, stream);
+    case 8: return taps_real ? launch_ptc_l<8, false, false>(a, smin, stream) : launch_ptc_l<8, true, false>(a, smin, stream);
+    case 4: return taps_real ? launch_ptc_l<4, false, false>(a, smin, stream) : launch_ptc_l<4, true, false>(a, smin, stream);
     default: set_error("fir_ptc: unsupported interpolation factor %u", seg.interp); return CB_ERR_UNSUPPORTED;
     }
 }

@@ -181,8 +181,11 @@ __device__ unsigned long long *g_ftc_dbg = nullptr;
 #endif
 
 // IQ16: the raw tiles are i16 IQ words (half the bytes; the first tile's halo is read from the f32 history by the
-// converters, a tile of 16-bit samples never needs the exact fall-back) and the epilogue writes i16 IQ words.
-template <int KB, int NRAW, bool IQ16 = false>
+// converters) and the epilogue writes i16 IQ words.  A tile of 16-bit samples never needs the exact fall-back, but the
+// first one's halo can hold anything (set_state, an f32 call): that tile takes the quiet test of the f32 form, so the
+// same tiles are recomputed and the words equal quantising the f32 result.
+// SMIN: the quiet test per sample (taps that may skip one sample of every pair, FirTcPlan::sample_min).
+template <int KB, int NRAW, bool IQ16 = false, bool SMIN = false>
 __global__ void __launch_bounds__(NTHREADS, 1) fir_tc_kernel(const __grid_constant__ Args a)
 {
     constexpr int HALO = RS * (KB - 1);            // complex samples of history per tile
@@ -331,6 +334,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) fir_tc_kernel(const __grid_consta
                         const long long g = t0 - HALO + 2 * q;  // even
                         if (q < NPAIR && (g < 0 || g + 1 >= ((long long)a.n & ~3ll))) raw[i] = iq16_edge_pair(a, g, HALO);
                     }
+                    if (t0 < HALO) {
+#pragma unroll
+                        for (int i = 0; i < NLD; ++i) {
+                            const float4 v = raw[i];
+                            mnu = min(mnu, quiet_key<SMIN>(v, fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w)))));
+                        }
+                    }
                 }
 #pragma unroll
                 for (int i = 0; i < NLD; ++i) {
@@ -354,7 +364,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) fir_tc_kernel(const __grid_consta
                     raw[i] = v;
                     const float pm = fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w)));
                     mx = fmaxf(mx, pm);
-                    mnu = min(mnu, __float_as_uint(pm) - 1u);
+                    mnu = min(mnu, quiet_key<SMIN>(v, pm));
                 }
             }
             mbar_arrive(&raw_empty[rs]);  // tile is in registers: the TMA warp may refill the stage
@@ -652,7 +662,7 @@ void fir_tc_build_image(const float2 *taps, uint32_t ntaps, unsigned char *img, 
     }
 }
 
-template <int KB, bool IQ16 = false>
+template <int KB, bool IQ16, bool SMIN>
 static int launch_tc_kb(const tc::Args &a, cudaStream_t stream)
 {
     constexpr int RAWB = (tc::TILE + tc::RS * (KB - 1)) * (IQ16 ? 4 : 8);
@@ -660,7 +670,7 @@ static int launch_tc_kb(const tc::Args &a, cudaStream_t stream)
     constexpr int NRAW = BASE + 2 * RAWB <= 227 * 1024 ? 2 : 1;
     constexpr int SMEM = BASE + NRAW * RAWB;
     static_assert(SMEM <= 227 * 1024, "fir_tc: shared memory budget");
-    auto kern = tc::fir_tc_kernel<KB, NRAW, IQ16>;
+    auto kern = tc::fir_tc_kernel<KB, NRAW, IQ16, SMIN>;
     CB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
     const unsigned long long ntiles = (a.n + tc::TILE - 1) / tc::TILE;
     int dev = 0, sms = 148;
@@ -693,64 +703,64 @@ bool fir_tc_iq16_applicable(const FirSeg &seg, const int16_t *x16, const int16_t
     return (reinterpret_cast<uintptr_t>(x16) & 15) == 0 && (reinterpret_cast<uintptr_t>(y16) & 3) == 0;
 }
 
-int launch_fir_tc_iq16(const FirSeg &seg, const int16_t *x16, float in_scale, int16_t *y16, float out_scale, const void *bimg_dev,
-                       float tap_inv_scale, cudaStream_t stream)
+// the kernel for the plan's tap count and quiet test, then the exact fall-back pass over the tiles it flagged
+static int launch_tc(const FirSeg &seg, tc::Args &a, bool iq16, const FirTcPlan &plan, const float2 *taps_dev,
+                     cudaStream_t stream)
 {
     if (seg.n_in == 0) return CB_OK;
     const int KB = fir_tc_kblocks(seg.ntaps);
-    tc::Args a = {};
     a.halo = seg.hist_in + (seg.hist_len - (uint32_t)tc::RS * (KB - 1));
     a.hist_in = seg.hist_in;
     a.hist_out = seg.hist_out;
-    a.bimg = reinterpret_cast<const uint4 *>(bimg_dev);
+    a.bimg = reinterpret_cast<const uint4 *>(plan.bimg_dev);
     a.n = seg.n_in;
     a.hist_len = seg.hist_len;
-    a.tap_inv_scale = tap_inv_scale;
-    a.x16 = reinterpret_cast<const uint32_t *>(x16);
-    a.y16 = reinterpret_cast<uint32_t *>(y16);
-    a.in_scale = in_scale;
-    a.out_scale = out_scale;
-    switch (KB) {
-    case 2: return launch_tc_kb<2, true>(a, stream);
-    case 3: return launch_tc_kb<3, true>(a, stream);
-    case 4: return launch_tc_kb<4, true>(a, stream);
-    case 5: return launch_tc_kb<5, true>(a, stream);
-    default: set_error("fir_tc: unsupported tap count %u", seg.ntaps); return CB_ERR_UNSUPPORTED;
-    }
-}
-
-int launch_fir_tc(const FirSeg &seg, const void *bimg_dev, float tap_inv_scale, FirFix *fix, const float2 *taps_dev,
-                  cudaStream_t stream)
-{
-    if (seg.n_in == 0) return CB_OK;
-    const int KB = fir_tc_kblocks(seg.ntaps);
-    tc::Args a = {};
-    a.x = seg.x;
-    a.halo = seg.hist_in + (seg.hist_len - (uint32_t)tc::RS * (KB - 1));
-    a.y = seg.y;
-    a.hist_in = seg.hist_in;
-    a.hist_out = seg.hist_out;
-    a.bimg = reinterpret_cast<const uint4 *>(bimg_dev);
-    a.n = seg.n_in;
-    a.hist_len = seg.hist_len;
-    a.tap_inv_scale = tap_inv_scale;
+    a.tap_inv_scale = plan.tap_inv_scale;
+    FirFix *fix = plan.fix;
     const bool fixup = fix != nullptr && fix->dev != nullptr && taps_dev != nullptr &&
                        fix->cap >= ceil_div(seg.n_in, (size_t)tc::TILE);
     a.fix_count = fixup ? fix->dev + (fix->calls & 1u) : nullptr;
     a.fix_list = fixup ? fix->dev + 2 : nullptr;
+    const int sel = KB * 4 + (iq16 ? 2 : 0) + (plan.sample_min ? 1 : 0);
     int rc;
-    switch (KB) {
-    case 2: rc = launch_tc_kb<2>(a, stream); break;
-    case 3: rc = launch_tc_kb<3>(a, stream); break;
-    case 4: rc = launch_tc_kb<4>(a, stream); break;
-    case 5: rc = launch_tc_kb<5>(a, stream); break;
+    switch (sel) {
+#define CB_TC_CASE(kb)                                                          \
+    case kb * 4 + 0: rc = launch_tc_kb<kb, false, false>(a, stream); break; \
+    case kb * 4 + 1: rc = launch_tc_kb<kb, false, true>(a, stream); break;  \
+    case kb * 4 + 2: rc = launch_tc_kb<kb, true, false>(a, stream); break;  \
+    case kb * 4 + 3: rc = launch_tc_kb<kb, true, true>(a, stream); break;
+    CB_TC_CASE(2)
+    CB_TC_CASE(3)
+    CB_TC_CASE(4)
+    CB_TC_CASE(5)
+#undef CB_TC_CASE
     default: set_error("fir_tc: unsupported tap count %u", seg.ntaps); return CB_ERR_UNSUPPORTED;
     }
     if (rc || !fixup) return rc;
-    FirFixArgs f{seg.x, seg.hist_in, taps_dev, seg.y, nullptr, 1.f, seg.n_in, seg.ntaps, 1u, (unsigned)tc::TILE, seg.hist_len,
-                 a.fix_count, fix->dev + ((fix->calls + 1) & 1u), a.fix_list};
+    FirFixArgs f{a.x, seg.hist_in, taps_dev, a.y, reinterpret_cast<int16_t *>(a.y16), a.out_scale, seg.n_in, seg.ntaps, 1u,
+                 (unsigned)tc::TILE, seg.hist_len, a.fix_count, fix->dev + ((fix->calls + 1) & 1u), a.fix_list, a.x16, a.in_scale};
     ++fix->calls;
     return launch_fir_fixup(f, stream);
+}
+
+int launch_fir_tc_iq16(const FirSeg &seg, const int16_t *x16, float in_scale, int16_t *y16, float out_scale,
+                       const FirTcPlan &plan, const float2 *taps_dev, cudaStream_t stream)
+{
+    tc::Args a = {};
+    a.x16 = reinterpret_cast<const uint32_t *>(x16);
+    a.y16 = reinterpret_cast<uint32_t *>(y16);
+    a.in_scale = in_scale;
+    a.out_scale = out_scale;
+    return launch_tc(seg, a, true, plan, taps_dev, stream);
+}
+
+int launch_fir_tc(const FirSeg &seg, const FirTcPlan &plan, const float2 *taps_dev, cudaStream_t stream)
+{
+    tc::Args a = {};
+    a.x = seg.x;
+    a.y = seg.y;
+    a.out_scale = 1.f;
+    return launch_tc(seg, a, false, plan, taps_dev, stream);
 }
 
 }  // namespace cb

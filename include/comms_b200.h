@@ -147,9 +147,13 @@ CB_API int cb_copy_d2h_async(void *dst_host, const void *src_dev, size_t bytes, 
  * zero-stuffed history (non-zero only every L-th entry, newest = index L-1
  * ... ) or be NULL; otherwise CB_ERR_UNSUPPORTED.
  */
-/* Numerical locality.  Filters of up to 128 taps (and the polyphase banks) keep the reference's locality exactly: a
- * quiet stretch next to a loud one keeps its own 1e-5, and an Inf / NaN input sample makes exactly the outputs
- * non-finite whose taps reach it (tiles the tensor-core kernels cannot hold to that are recomputed in plain f32).  The
+/* Numerical locality.  Filters of up to 128 taps (and the polyphase banks) keep the reference's locality per output:
+ * every output y[n] is within 1e-5 * sum_k |taps[k]| |x[n-k]| of the exact value -- a quiet stretch next to a loud
+ * one keeps its own accuracy -- and an Inf / NaN input sample makes exactly the outputs non-finite whose taps reach it
+ * (tiles the tensor-core kernels cannot hold to that are recomputed in plain f32).  One exception: the tensor-core
+ * kernels split the taps with one scale, so a tap far below the largest is carried to ~2^-39 of the largest tap in
+ * absolute terms (an impulse through a tap of 1e-8 of the largest is off by ~1e-4 of itself); with any dense input
+ * this is far below f32 rounding.  The
  * fast-convolution path for 129..1025 taps (calls of >= 8192 samples) works on frames of 4096 points: its error is
  * relative to the frame's energy (~4e-7 of it), and one non-finite sample makes the ~3000 outputs of its frame
  * non-finite.  COMMS_B200_FIR_PATH=cuda selects the direct form for such filters when that matters. */

@@ -66,8 +66,9 @@ int main(int argc, char **argv)
     cudaEventCreate(&e1);
     for (int it = 0; it < 3; ++it) {
         cudaEventRecord(e0);
-        int rc = iq16 ? cb::launch_fir_tc_iq16(seg, reinterpret_cast<const int16_t *>(x), 1.f / 32768, reinterpret_cast<int16_t *>(y), 8192.f, img, tis, 0)
-                      : cb::launch_fir_tc(seg, img, tis, nullptr, nullptr, 0);
+        const cb::FirTcPlan plan{img, tis, 1};
+        int rc = iq16 ? cb::launch_fir_tc_iq16(seg, reinterpret_cast<const int16_t *>(x), 1.f / 32768, reinterpret_cast<int16_t *>(y), 8192.f, plan, nullptr, 0)
+                      : cb::launch_fir_tc(seg, plan, nullptr, 0);
         if (rc) return 1;
         cudaEventRecord(e1);
         if (cudaDeviceSynchronize() != cudaSuccess) { fprintf(stderr, "kernel failed: %s\n", cudaGetErrorString(cudaGetLastError())); return 1; }
