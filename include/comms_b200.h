@@ -155,8 +155,10 @@ CB_API int cb_copy_d2h_async(void *dst_host, const void *src_dev, size_t bytes, 
  * absolute terms (an impulse through a tap of 1e-8 of the largest is off by ~1e-4 of itself); with any dense input
  * this is far below f32 rounding.  The
  * fast-convolution path for 129..1025 taps (calls of >= 8192 samples) works on frames of 4096 points: its error is
- * relative to the frame's energy (~4e-7 of it), and one non-finite sample makes the ~3000 outputs of its frame
- * non-finite.  COMMS_B200_FIR_PATH=cuda selects the direct form for such filters when that matters. */
+ * relative to the frame's energy: every output of frame f is within (2 rho_4096 + 2^-24) * max_k |H_k| * ||x_f||_2
+ * of the exact value (rho_4096 = 1.6 * 12 * 2^-24, the FFT's norm bound below; H the 4096-point transform of the taps;
+ * x_f the frame's 4096 inputs, history included), and one non-finite sample makes the outputs of exactly the frames
+ * whose 4096 inputs hold it non-finite.  COMMS_B200_FIR_PATH=cuda selects the direct form for such filters when that matters. */
 CB_API int cb_fir_create(const float *taps, size_t ntaps, const float *state, size_t nstate,
                          uint32_t decim, uint32_t interp, cb_fir **out);
 CB_API int cb_fir_destroy(cb_fir *h);
@@ -232,7 +234,16 @@ CB_API int cb_mixer_set_phase(cb_mixer *h, double phase);
  * beyond that cb_fft_create returns CB_ERR_UNSUPPORTED.
  * n_in must be a multiple of fft_size (the reference requires n_in ==
  * fft_size, one frame per message; several contiguous frames per call is the
- * batched form) else CB_ERR_SIZE. */
+ * batched form) else CB_ERR_SIZE.
+ * Numerical contract, per frame f of N points with S_f = sum_n |x[n]|, u = 2^-24 and X the exact transform: every
+ * bin satisfies |X'[k] - X[k]| <= tau * S_f (+ 4 N 2^-149 for subnormal frames) and the frame
+ * ||X' - X||_2 <= rho * ||X||_2, with
+ *   powers of two (8 .. 2^20):       tau = 4 log2(N) u,    rho = 1.6 log2(N) u  (<= 2e-6 at every size)
+ *   direct O(N^2) sums (N <= 128):   tau = rho = 5 u, whatever N
+ *   chirp-z (M = padded power of two, the least >= max(256, 2N - 1)):
+ *                                    tau = 5.4 log2(M) u,  rho = 2 log2(M) u.
+ * A frame of zeros gives exact zeros.  A non-finite input makes every bin of its own frame non-finite and no other:
+ * the other frames of the batch keep their bounds (tests/test_gpu_fft_bounds.py checks every bin of every plan). */
 CB_API int cb_fft_create(size_t fft_size, int inverse, cb_fft **out);
 CB_API int cb_fft_destroy(cb_fft *h);
 CB_API int cb_fft_run(cb_fft *h, const float *in, size_t n_in, float *out);

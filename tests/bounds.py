@@ -179,3 +179,173 @@ def parity_sparse(taps):
     nz = np.abs(np.asarray(taps)) != 0
     adj = nz[1:] & nz[:-1]  # adj[i]: taps i and i + 1 both non-zero, the pair ends at offset i + 1
     return bool(nz.any()) and not (adj[1::2].any() and adj[0::2].any())
+
+
+# ---------------------------------------------------------------------------------------------------------------- FFT
+# Every bin X_k = sum_n x_n W^{kn} is a sum over all inputs with unit-modulus twiddles, so its rounding error scales
+# with S_f = sum_n |x_n| of its frame, not with |X_k| nor with the frame's norm.  Checked, for EVERY bin of EVERY
+# frame of an N-point transform computed in f32 (u = 2^-24):
+#
+#     |got_k - X_k| <= tau * S_f + FFT_FLOOR * N * 2^-149      and      ||got_f - X_f||_2 <= rho ||X_f||_2 (+ floor)
+#
+#   power-of-two sizes (radix 16 passes, two-step splits):  tau = C_TAU log2(N) u,  rho = C_RHO log2(N) u
+#   direct O(N^2) sum (N <= 128 otherwise):                  tau = rho = C_DIRECT u, whatever N
+#   chirp-z (any other N, M = padded power of two):           tau = C_CHIRPZ log2(M) u,  rho = C_CHIRPZ_RHO log2(M) u
+#
+# with X the complex128 transform.  Exact cases: a frame with S_f = 0 gives exact zeros; a frame holding a non-finite
+# input gives every bin non-finite (in at least one component), and every other frame of the batch stays finite and
+# within its bounds.
+#
+# The constants are twice (at most) the worst ratio seen in the CPU emulation of the device arithmetic
+# (tests/emul/fft2_emul.cpp; tests/test_fft_bounds_cpu.py checks them):
+# - C_TAU: an impulse is the worst case, every output being a product of rounded twiddles.  The twiddle16 power tree
+#   (depth 4), the bfly16 constant rotations and the table entries each add a rounding per 16-point digit: worst
+#   emulated 2.05 (65536 points, 256 x 256 with twiddle16c), 1.88 (4096), 1.64 (256).
+# - C_RHO: worst emulated 0.96 (a tone on an exact bin, 4096-point inverse); random frames 0.3 .. 0.53.  1.6 keeps
+#   rho <= 2e-6 up to 2^20 points.
+# - C_DIRECT: dft_direct_kernel multiplies by an exact-angle table entry (|dw| <= 0.71 u), rounds the complex
+#   product (normwise <= 2 u |x_n| with the fused multiply-add, Jeannerod et al. 2017) and sums with Kahan
+#   compensation (<= 2 u sum |terms| + O(N u^2) S_f = 2 u S_f): (0.71 + 2 + 2) u S_f, rounded up to 5 u S_f.
+# - C_CHIRPZ, C_CHIRPZ_RHO: the emulation also runs the fused chirp-z kernel (bluestein_frames_kernel) on the same
+#   passes, M = 512 .. 16384, with the chirp and its f32-rounded spectrum B exactly as bluestein_setup builds them.
+#   It meets the S_f form with log2(M): worst 2.74 (impulses, N = 4095), norm 1.00 (random frames, N = 8191).  The
+#   worst-case algebra would let the error grow with sqrt(N) (the inverse transform's input has sum |Z_k| ~
+#   M sqrt(2N) |x|); neither this emulation nor a NumPy f32 emulation of the sequence up to M = 2^20 shows growth.
+FFT_U = 2.0 ** -24
+C_TAU = 4.0
+C_RHO = 1.6
+C_DIRECT = 5.0
+C_CHIRPZ = 5.4
+C_CHIRPZ_RHO = 2.0
+FFT_FLOOR = 4.0  # absolute floor, in units of N * 2^-149 (chirp-z: M sqrt(2N) * 2^-149): subnormal frames
+
+
+def chirpz_m(n):
+    """padded size of the chirp-z plan: the least power of two >= max(256, 2N - 1) (bluestein_setup, api.cu)"""
+    m = 256
+    while m < 2 * n - 1:
+        m <<= 1
+    return m
+
+
+def fft_path(n, direct=False):
+    """the kind of plan cb_fft_create makes for N points: 'pow2' (2^3 .. 2^20), 'direct' (any other N <= 128, or up
+    to 4096 with COMMS_B200_FFT_PATH=direct) or 'chirpz'"""
+    if n >= 8 and n & (n - 1) == 0:
+        return "pow2"
+    return "direct" if n <= 128 or (direct and n <= 4096) else "chirpz"
+
+
+def fft_constants(n, path):
+    """(tau, rho, floor) of an N-point transform on `path`: |err_k| <= tau S_f + floor, ||err|| <= rho ||X|| +
+    floor sqrt(N)"""
+    if path == "direct":
+        return C_DIRECT * FFT_U, C_DIRECT * FFT_U, FFT_FLOOR * n * 2.0 ** -149
+    if path == "chirpz":
+        m = chirpz_m(n)
+        lm = np.log2(m)
+        return C_CHIRPZ * lm * FFT_U, C_CHIRPZ_RHO * lm * FFT_U, FFT_FLOOR * m * np.sqrt(2 * n) * 2.0 ** -149
+    assert path == "pow2", path
+    return C_TAU * np.log2(n) * FFT_U, C_RHO * np.log2(n) * FFT_U, FFT_FLOOR * n * 2.0 ** -149
+
+
+def fft64(x, n, inverse=False):
+    """the product's unnormalised transform of every frame in complex128 (frames, n): X_k = sum x_n e^{-/+ 2 pi i kn/N}"""
+    x = np.asarray(x).astype(np.complex128).reshape(-1, n)
+    with np.errstate(all="ignore"):
+        return np.fft.ifft(x, axis=1) * n if inverse else np.fft.fft(x, axis=1)
+
+
+def fft_bound_report(got, x, n, inverse=False, path=None, exact=None):
+    """Check every bin of every frame.  Returns (failures, worst bin ratio, worst norm ratio): failures is a list of
+    messages naming the frame, the bin and the ratio; the ratios are over the finite frames with S_f > 0, as
+    |err_k| / bin bound and ||err|| / norm bound (<= 1 passes).  `exact`: fft64(x, n, inverse) if already at hand."""
+    path = path or fft_path(n)
+    tau, rho, floor = fft_constants(n, path)
+    x = np.asarray(x).reshape(-1, n)
+    g = np.asarray(got).reshape(-1, n).astype(np.complex128)
+    assert g.shape == x.shape, (g.shape, x.shape)
+    X = fft64(x, n, inverse) if exact is None else np.asarray(exact).reshape(-1, n)
+    xa = np.abs(x.astype(np.complex128))
+    finite_in = np.isfinite(x.real).all(axis=1) & np.isfinite(x.imag).all(axis=1)
+    with np.errstate(all="ignore"):
+        S = xa.sum(axis=1)
+        gfin = np.isfinite(g.real) & np.isfinite(g.imag)
+        err = np.abs(g - X)
+        bb = tau * S + floor
+        rbin = err / bb[:, None]
+        enorm = np.sqrt((err ** 2).sum(axis=1))
+        nb = rho * np.sqrt((np.abs(X) ** 2).sum(axis=1)) + floor * np.sqrt(n)
+        rnorm = enorm / nb
+    fails, wbin, wnorm = [], 0.0, 0.0
+    where = f"{path} N={n} {'inverse' if inverse else 'forward'}"
+    for f in range(x.shape[0]):
+        if not finite_in[f]:
+            ok = ~gfin[f]
+            if not ok.all():
+                k = int(np.argmin(ok))
+                fails.append(f"{where}: frame {f} holds a non-finite input but bin {k} is finite ({g[f, k]}); "
+                             f"{int((~ok).sum())} of {n} bins finite")
+            continue
+        if not gfin[f].all():
+            k = int(np.argmin(gfin[f]))
+            fails.append(f"{where}: frame {f} (finite input) has non-finite bin {k} ({g[f, k]}); "
+                         f"{int((~gfin[f]).sum())} of {n} bins non-finite")
+            continue
+        if S[f] == 0:
+            if np.any(g[f] != 0):
+                k = int(np.argmax(g[f] != 0))
+                fails.append(f"{where}: frame {f} is all zeros but bin {k} is {g[f, k]} "
+                             f"({int((g[f] != 0).sum())} of {n} bins non-zero)")
+            continue
+        k = int(np.argmax(rbin[f]))
+        wbin, wnorm = max(wbin, float(rbin[f, k])), max(wnorm, float(rnorm[f]))
+        if rbin[f, k] > 1:
+            fails.append(f"{where}: frame {f} bin {k}: |err|/bound = {rbin[f, k]:.3g} ({int((rbin[f] > 1).sum())} of "
+                         f"{n} bins outside), got {g[f, k]}, exact {X[f, k]}, bound {bb[f]:.3g}")
+        if rnorm[f] > 1:
+            fails.append(f"{where}: frame {f}: ||err||/(rho ||X||) = {rnorm[f]:.3g} (rho {rho:.3g})")
+    return fails, wbin, wnorm
+
+
+def assert_fft_bound(got, x, n, inverse=False, path=None, what="", exact=None):
+    """every bin of every frame within its bound (see fft_bound_report); returns the worst (bin, norm) ratios"""
+    fails, wbin, wnorm = fft_bound_report(got, x, n, inverse, path, exact)
+    assert not fails, f"{what}: {len(fails)} failures; " + "; ".join(fails[:6])
+    return wbin, wnorm
+
+
+# ---------------------------------------------------------------------------------------------------- overlap-save FIR
+OLS_N = 4096
+
+
+def ols_bound(x, taps, hist=None):
+    """Per-output bound of the overlap-save FIR (fir_ols_kernel, 4096-point frames, hop 4097 - K) for one call of
+    x after the newest-first history `hist` (None: zeros): output n comes from frame f = n // hop, whose inputs are
+    x_f = samples [f hop - (K - 1), f hop - (K - 1) + 4096) of the call (history before 0, zeros past the call's end).
+    Forward transform, product with Hf and inverse each obey the FFT norm bound, so
+
+        |err_n| <= (2 rho_4096 + u) ||H||_inf ||x_f||_2,   H = 4096-point DFT of the taps in float64 from the f32 taps.
+
+    Returns (bound per output, frame index per output)."""
+    t = np.asarray(taps, np.complex64).astype(np.complex128)
+    K = len(t)
+    hop = OLS_N - (K - 1)
+    x = np.asarray(x).astype(np.complex128)
+    h = np.zeros(K - 1, np.complex128) if hist is None else np.asarray(hist, np.complex128)[: K - 1][::-1]
+    full = np.concatenate([np.zeros(K - 1 - len(h), np.complex128), h, x, np.zeros(OLS_N, np.complex128)])
+    H = np.fft.fft(np.concatenate([t, np.zeros(OLS_N - K)]))
+    frames = -(-len(x) // hop)
+    win = np.lib.stride_tricks.sliding_window_view(np.abs(full), OLS_N)[::hop][:frames]  # index 0: sample -(K - 1)
+    with np.errstate(all="ignore"):
+        xn = np.sqrt((win ** 2).sum(axis=1))
+    _, rho, _ = fft_constants(OLS_N, "pow2")
+    f = np.arange(len(x)) // hop
+    return (2 * rho + FFT_U) * np.abs(H).max() * xn[f], f
+
+
+def ols_seams(n, ntaps):
+    """first and last output of every overlap-save frame of an n-sample call"""
+    hop = OLS_N - (ntaps - 1)
+    s = np.arange(0, n, hop)
+    return np.unique(np.clip(np.concatenate([s - 1, s]), 0, n - 1))
