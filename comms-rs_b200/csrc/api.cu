@@ -2578,6 +2578,8 @@ static int freq_estimate_impl(const double2 *samples, bool on_host, size_t n, do
         return CB_OK;
     }
     CB_REQUIRE(samples, CB_ERR_INVALID_ARG, "NULL data pointer");
+    CB_REQUIRE(on_host || (reinterpret_cast<uintptr_t>(samples) & 15) == 0, CB_ERR_INVALID_ARG,
+               "frequency estimator: d_samples must be 16-byte aligned");  // read as double2
     int rc = ensure_device();
     if (rc) return rc;
     EstScratch sc;
@@ -2661,6 +2663,8 @@ static int timing_push_impl(cb_timing *h, const double2 *samples, bool on_host, 
     double2 sum = make_double2(0.0, 0.0);
     if (n > 0) {
         CB_REQUIRE(samples, CB_ERR_INVALID_ARG, "NULL data pointer");
+        CB_REQUIRE(on_host || (reinterpret_cast<uintptr_t>(samples) & 15) == 0, CB_ERR_INVALID_ARG,
+                   "timing estimator: d_samples must be 16-byte aligned");  // read as double2
         CB_CUDA(cudaSetDevice(h->device));
         EstScratch sc;
         int rc = sc.alloc(s, on_host ? n : 0);

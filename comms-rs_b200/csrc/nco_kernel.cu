@@ -87,6 +87,10 @@ __global__ void __launch_bounds__(1024) nco_scan_tiles_kernel(double *__restrict
             const double t = __shfl_up_sync(0xffffffffu, incl, o);
             if ((threadIdx.x & 31) >= o) incl += t;
         }
+        // exclusive prefix by shifting the inclusive scan up one lane, never as incl - v: a non-finite or huge tile sum
+        // must not reach the prefixes of the tiles before it
+        double excl = __shfl_up_sync(0xffffffffu, incl, 1);
+        if ((threadIdx.x & 31) == 0) excl = 0.0;
         if ((threadIdx.x & 31) == 31) ws[threadIdx.x >> 5] = incl;
         __syncthreads();
         if (threadIdx.x < 32) {
@@ -101,7 +105,7 @@ __global__ void __launch_bounds__(1024) nco_scan_tiles_kernel(double *__restrict
         __syncthreads();
         const double before_warp = (threadIdx.x >> 5) ? ws[(threadIdx.x >> 5) - 1] : 0.0;
         const double carry = carry_s;
-        if (i < ntiles) tile_sum[i] = reduce_2pi(carry + before_warp + (incl - v), 0.0);
+        if (i < ntiles) tile_sum[i] = reduce_2pi(carry + before_warp + excl, 0.0);
         __syncthreads();
         if (threadIdx.x == 1023) carry_s = reduce_2pi(carry + before_warp + incl, 0.0);
         __syncthreads();
@@ -129,16 +133,19 @@ __global__ void __launch_bounds__(NCO_THREADS) nco_apply_kernel(const double *__
     }
 #pragma unroll
     for (int i = 1; i < NCO_PER_THREAD; ++i) v[i] += v[i - 1];  // thread-local inclusive scan
-    const double mine = v[NCO_PER_THREAD - 1];
-    double incl = mine;
+    double incl = v[NCO_PER_THREAD - 1];
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
         const double t = __shfl_up_sync(0xffffffffu, incl, o);
         if ((threadIdx.x & 31) >= o) incl += t;
     }
+    // exclusive prefix of the lanes before this one (shifted scan, not incl - mine: output k depends on perr[0..k] only,
+    // so a NaN, an Inf or one huge value cannot change or cancel into the outputs before it)
+    double excl = __shfl_up_sync(0xffffffffu, incl, 1);
+    if ((threadIdx.x & 31) == 0) excl = 0.0;
     if ((threadIdx.x & 31) == 31) ws[threadIdx.x >> 5] = incl;
     __syncthreads();
-    double off = tile_pre[blockIdx.x] + (incl - mine);
+    double off = tile_pre[blockIdx.x] + excl;
     for (int w = 0; w < (int)(threadIdx.x >> 5); ++w) off += ws[w];
     const double ph0 = *phase_in;
 #pragma unroll

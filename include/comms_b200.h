@@ -218,7 +218,13 @@ CB_API int cb_upsample(const void *in, size_t n, size_t elem_bytes, size_t rate,
  * Replaces Mixer::new / Mixer::mix (src/mixer.rs:43-51, :73-84) over a batch:
  *   y[n] = x[n] * exp(j*(phase + n*dphase)),  dphase wrapped into [0, 2pi)
  * Phase arithmetic in f64, carried across calls.  Note the argument order of
- * MixerNode::new(dphase, phase) (src/mixer.rs:128). */
+ * MixerNode::new(dphase, phase) (src/mixer.rs:128).
+ * Accuracy, every output n counted from the stream's start (u32 = 2^-24, u64 = 2^-53, theta_n the exact phase):
+ *   |y[n] - x[n] exp(j theta_n)| <= (13 u32 + u64 (|phase| + n dphase + 8 pi + c)) |x[n]| + 2^-148,
+ * with c = sum over earlier calls of (2 pi + 2^-9 (|phase entering the call| + its length * dphase)) for the carried
+ * phase.  13 u32 comes from sincosf's 2 ulp, the hi/lo correction and two fused complex products.  x[n] = 0 gives an
+ * exact 0; a non-finite x[n] gives a non-finite y[n] and leaves every other output unchanged.
+ * (tests/test_gpu_phase_bounds.py checks every output.) */
 CB_API int cb_mixer_create(double dphase, double phase, cb_mixer **out);
 CB_API int cb_mixer_destroy(cb_mixer *h);
 CB_API int cb_mixer_run(cb_mixer *h, const float *in, size_t n, float *out);
@@ -335,11 +341,21 @@ CB_API int cb_quantize_i16_dev(const float *d_in, size_t nfloats, float scale, i
  * The two feed-forward estimators of src/demodulation that call batch_fir (complex f64 samples = 2n interleaved
  * doubles).  Each call is one fused pass (filter, product, reduction) and returns its scalar on the host, so it
  * synchronises the stream it ran on.
+ * d_samples of the _dev forms must be 16-byte aligned (read as pairs of doubles); other pointers return
+ * CB_ERR_INVALID_ARG before any launch.
  * cb_freq_estimate: frequency_offset_estimate (src/demodulation/frequency_estimator.rs:27-42), radians/sample:
  *   arg(sum_{i<n-1} x[i+1] conj(x[i])); n < 2 gives 0.
+ *   Accuracy: |est - arg S| <= asin(E / |S|) + 2^-49 (S the exact sum) whenever E < |S|, with
+ *   E = sqrt(2) u64 D sum |x[i+1]| |x[i]|, D = m + ceil(P / 256) + 26, P = min(ceil(n / 2048), 1184) CTAs and
+ *   m = ceil((n - 1) / (256 P)) terms per thread.  When E >= |S| the estimate is finite but carries no guarantee.
+ *   A NaN sample gives NaN.
  * cb_timing_*: TimingEstimator::new / push (src/demodulation/timing_estimator.rs:43-58, 85-112), result in
  *   samples; alpha outside [0, 1] -> CB_ERR_INVALID_ARG (MathError::InvalidRolloffError); the internal filter
  *   length 2*n*d+1 is limited to 4097 (CB_ERR_UNSUPPORTED beyond).
+ *   Accuracy: |est - est_exact| <= (n / 2 pi) (asin(E / |S|) + 2^-49) whenever E < |S|, S = sum_i qout_i dout_i exact
+ *   (the reference's r_m = exp(-j fl(fl(-pi m) / n)) argument), E = u64 (sqrt(2) (ntaps4 + D) + 16) sum_i |dout_i| A_i,
+ *   A_i = sum_k |q_k| |qin_{i-k}|, ntaps4 = the tap count rounded up to four, D = 4 ceil(T / P) + ceil(P / 256) + 26
+ *   for T = ceil(len / 1024) tiles over P = min(T, 1184) CTAs.
  * cb_qfilt_taps_f64: qfilt_taps (src/util/math.rs:307-342); taps must hold n_taps + 1 doubles (an even n_taps is
  *   incremented by one); *n_out receives the count written. */
 typedef struct cb_timing cb_timing;
@@ -357,7 +373,13 @@ CB_API int cb_timing_push_dev(cb_timing *h, const double *d_samples, size_t n, d
  * i.e. phase_k = phase_0 + (k+1)*dphase + sum_{i<=k} perr[i] (mod 2 pi): a prefix sum, evaluated as a device scan in
  * f64 with the ramp term reduced exactly; the wrap only picks the representative of the phase, never the output.
  * n doubles in -> n complex f64 (2n doubles) out; dphase wrapped into [0, 2 pi) like Nco::new; phase carried across
- * calls (cb_nco_get_phase returns it reduced to [0, 2 pi)).  At most 2^29 - 1 errors per call. */
+ * calls (cb_nco_get_phase returns it reduced to [0, 2 pi)).  At most 2^29 - 1 errors per call.
+ * Accuracy, causal: output k depends on perr[0..k] only, and
+ *   |out[k] - exp(j phi_k)| <= u64 (2 (|phase_0| + 2 pi (1 + calls_k + chunks_k)) + 16 S_k + 6),
+ * phi_k the exact phase from the stream's start (or from the last cb_nco_set_phase, phase_0 its phase),
+ * S_k = sum_{i<=k} |perr[i]|, calls_k = calls before the one holding k, chunks_k = (k within its call) / 2^21.
+ * A NaN or infinite perr[j] makes out[j..] and the carried phase NaN, as in the reference recurrence; out[0..j-1]
+ * keep the bound.  A huge perr[j] enters the bound of out[j..] only. */
 typedef struct cb_nco cb_nco;
 CB_API int cb_nco_create(double dphase, double phase, cb_nco **out);
 CB_API int cb_nco_destroy(cb_nco *h);

@@ -349,3 +349,366 @@ def ols_seams(n, ntaps):
     hop = OLS_N - (ntaps - 1)
     s = np.arange(0, n, hop)
     return np.unique(np.clip(np.concatenate([s - 1, s]), 0, n - 1))
+
+
+# ------------------------------------------------------------------------------------ phase laws: mixer, NCO, estimators
+# References for the kernels whose output is a phase law (the stand-alone mixer, the NCO scan) and for the two f64
+# estimators, with the per-output bounds that include/comms_b200.h states.  u32 = 2^-24, u64 = 2^-53.
+#
+# The exact phase is formed in double-double: k * dphase as a Dekker two-product, phase0 and the prefix of perr added
+# with two-sums, and the result reduced against a three-part 2 pi (159 bits, from the integer below) with two-products
+# for q * P1 and q * P2.  For |theta| < 2^33 the reduced phase is correct to about 2^-72 rad; it is then handed to
+# long double (64-bit mantissa: 2^-64 pi) for sin and cos.  np.longdouble is NOT used for the reduction: its 64-bit
+# 2 pi would be off by about 1e-10 rad at k * dphase ~ 2^32.
+U32 = 2.0 ** -24
+U64 = 2.0 ** -53
+TWO_PI_2_200 = 10096689509235987743946820282484873672429286842977325943070736  # floor(2 pi 2^200)
+
+
+def _two_pi_parts():
+    from fractions import Fraction
+    t = Fraction(TWO_PI_2_200, 1 << 200)
+    p1 = float(t)
+    p2 = float(t - Fraction(p1))
+    p3 = float(t - Fraction(p1) - Fraction(p2))
+    return p1, p2, p3
+
+
+TWO_PI_P1, TWO_PI_P2, TWO_PI_P3 = _two_pi_parts()
+
+
+def two_sum(a, b):
+    s = a + b
+    bb = s - a
+    return s, (a - (s - bb)) + (b - bb)
+
+
+def _split(a):
+    c = 134217729.0 * a  # 2^27 + 1
+    hi = c - (c - a)
+    return hi, a - hi
+
+
+def two_prod(a, b):
+    """(p, e) with p + e = a * b exactly (Dekker; NumPy does not contract to FMA)"""
+    a, b = np.asarray(a, np.float64), np.asarray(b, np.float64)
+    p = a * b
+    ah, al = _split(a)
+    bh, bl = _split(b)
+    return p, ((ah * bh - p) + ah * bl + al * bh) + al * bl
+
+
+def dd_add(ah, al, bh, bl):
+    s, e = two_sum(ah, bh)
+    e = e + (al + bl)
+    return two_sum(s, e)
+
+
+def phase_exact(phase0, dphase, k, prefix=None):
+    """theta = phase0 + k dphase + prefix reduced mod 2 pi into about [-pi, pi], as a double-double (hi, lo).
+    k: integer array (k < 2^29); prefix: None, an array of doubles, or a (hi, lo) pair of arrays (exact sums)."""
+    with np.errstate(all="ignore"):
+        k = np.asarray(k, np.float64)
+        h, l = two_prod(k, np.float64(dphase))
+        h, l = dd_add(h, l, np.float64(phase0), 0.0)
+        if prefix is not None:
+            ph, pl = prefix if isinstance(prefix, tuple) else (np.asarray(prefix, np.float64), 0.0)
+            h, l = dd_add(h, l, ph, pl)
+        q = np.rint(h / TWO_PI_P1)
+        q = np.where(np.isfinite(q), q, 0.0)
+        a, b = two_prod(q, TWO_PI_P1)
+        h, l = dd_add(h, l, -a, -b)
+        a, b = two_prod(q, TWO_PI_P2)
+        h, l = dd_add(h, l, -a, -b)
+        h, l = dd_add(h, l, -q * TWO_PI_P3, 0.0)
+    return h, l
+
+
+def _cis_ld(h, l):
+    """(cos, sin) of the double-double phase, in long double"""
+    t = np.asarray(h).astype(np.longdouble) + np.asarray(l).astype(np.longdouble)
+    return np.cos(t), np.sin(t)
+
+
+def _err_ld(got, c, s):
+    """|got - (c + j s)| with the reference kept in long double"""
+    g = np.asarray(got).astype(np.complex128)
+    with np.errstate(all="ignore"):
+        dr = g.real.astype(np.longdouble) - c
+        di = g.imag.astype(np.longdouble) - s
+        return np.sqrt(dr * dr + di * di).astype(np.float64)
+
+
+# ---- mixer: y_n = x_n e^{j theta_n}, theta_n = phase + n dphase, carried across calls
+# The f64 part (fma(i, dphase, phase0) and the Cody-Waite reduction) rounds once at |theta|: u64 (|phase0| + n dphase)
+# rad.  The f32 part rests on sincosf's documented maximum error of 2 ulp (CUDA programming guide, Table of
+# single-precision functions), so it is derived rather than emulated: per component 2 u32 (sincosf) + u32 (the fmaf of
+# the hi/lo correction) + the second-order term lo^2/2 < 2^-47, i.e. |r - e^{j theta}| <= 3 sqrt(2) u32 for one
+# rotation; the vector path's r_k = r0 s_k adds a second rotation and a fused complex product (2 u32, Jeannerod et al.
+# 2017); the final x r adds 2 u32 |x|: 2 (3 sqrt 2) + 2 + 2 = 12.5, rounded up to C_MIX = 13.  Subnormal outputs add
+# an absolute floor of 2^-148 (two roundings at 2^-150 per component).  The carried phase (advance_phase, api.cu)
+# rounds once to f64 per call (u64 2 pi) after a long double fmodl whose 2 pi is off by 2 pi 2^-64 per turn.
+C_MIX = 13.0
+MIX_FLOOR = 2.0 ** -148
+
+
+def mix_exact(x, dphase, phase0, start=0):
+    """(cos, sin) of the exact phase for the samples start .. start + len(x) of a stream whose sample 0 had phase
+    phase0 (dphase as the handle holds it), and the exact x e^{j theta} in long double (re, im)"""
+    k = start + np.arange(len(x), dtype=np.int64)
+    c, s = _cis_ld(*phase_exact(phase0, dphase, k))
+    xr = np.asarray(x).real.astype(np.longdouble)
+    xi = np.asarray(x).imag.astype(np.longdouble)
+    return xr * c - xi * s, xr * s + xi * c
+
+
+def mix_carry(phase_in, m, dphase):
+    """what one call of m samples adds to the `carried` term: the f64 rounding of the carried phase (2 pi) and the long
+    double steps of advance_phase (2^-64 (|phase_in| + m dphase) each, with a 64-bit 2 pi), in units of u64"""
+    return 2 * np.pi + 2.0 ** -9 * (abs(phase_in) + m * dphase)
+
+
+def mix_bound(x, dphase, phase0, start=0, carried=0.0):
+    """per-output bound (C_MIX u32 + u64 (|phase0| + n dphase + 8 pi + carried)) |x_n| + MIX_FLOOR, n counted from the
+    stream's start; 8 pi covers the rounding of 2 dphase, 3 dphase and the quad's first phase; `carried`: the sum of
+    mix_carry over the calls before this one"""
+    n = start + np.arange(len(x), dtype=np.float64)
+    return (C_MIX * U32 + U64 * (abs(phase0) + n * dphase + 8 * np.pi + carried)) * np.abs(
+        np.asarray(x).astype(np.complex128)) + MIX_FLOOR
+
+
+def mix_bound_report(got, x, dphase, phase0, start=0, carried=0.0, idx=None):
+    """(failures, worst index, worst ratio): every output within mix_bound; a zero input gives an exact zero; a
+    non-finite input gives a non-finite output (in at least one component); finite inputs give finite outputs"""
+    g = np.asarray(got).astype(np.complex128)
+    x = np.asarray(x).astype(np.complex128)
+    fin_x = np.isfinite(x.real) & np.isfinite(x.imag)
+    xs = np.where(fin_x, x, 0)
+    er, ei = mix_exact(xs, dphase, phase0, start)
+    with np.errstate(all="ignore"):
+        dr = g.real.astype(np.longdouble) - er
+        di = g.imag.astype(np.longdouble) - ei
+        err = np.sqrt(dr * dr + di * di).astype(np.float64)
+        r = err / mix_bound(xs, dphase, phase0, start, carried)
+    fin_g = np.isfinite(g.real) & np.isfinite(g.imag)
+    r = np.where(fin_x, np.where(fin_g, r, np.inf), np.where(fin_g, np.inf, 0.0))
+    r = np.where(fin_x & (x == 0), np.where(g == 0, 0.0, np.inf), r)
+    if idx is not None:
+        keep = np.zeros(len(r), bool)
+        keep[np.asarray(idx, np.int64)] = True
+        r = np.where(keep, r, 0.0)
+    bad = np.nonzero(r > 1)[0]
+    w = int(np.argmax(r)) if len(r) else 0
+    fails = [f"mixer output {int(bad[0]) + start} (stream index): |err|/bound = {r[bad[0]]:.3g}, got {g[bad[0]]}, "
+             f"x {x[bad[0]]}; {len(bad)} outputs outside"] if len(bad) else []
+    return fails, w, float(r[w]) if len(r) else 0.0
+
+
+# ---- NCO: out_k = e^{j phi_k}, phi_k = phase_0 + (k + 1) dphase + sum_{i <= k} perr_i (mod 2 pi), carried
+# Causal bound (only perr[0..k] enters the bound of output k):
+#
+#     |out_k - e^{j phi_k}| <= u64 (C_NCO_A (|phase_0| + 2 pi (1 + calls_k + chunks_k)) + C_NCO_B S_k + C_SINCOS)
+#
+# S_k = sum_{i <= k} |perr_i| over the stream, calls_k = calls before the one holding k (each re-reduces the carried
+# phase), chunks_k = scan chunks of 2^21 samples before k in its call (each re-reduces the carry).  C_NCO_A and
+# C_NCO_B are twice (at most) the worst ratios of the CPU emulation of the device's f64 operation sequence
+# (tests/emul/phase_emul.cpp, checked in tests/test_phase_bounds_cpu.py): 0.52 of the bound with phase_0 = 1e6 + 0.3
+# (ph0 + reduce(...) + (off + v) rounds twice at |phase_0|), 0.56 with perr = 1 at each thread's first sample and 2^-53 (1 + 2^-20) elsewhere
+# (every addition of the thread, warp and CTA scans rounds the same way), 0.11 on random perr over three scan chunks.
+# C_SINCOS: the device's f64 sincos is within 2 ulp per component (CUDA programming guide): 2 ulp(1) sqrt 2 = 4 sqrt
+# 2 u64, rounded up to 6.  A non-finite perr_j makes out_j.., and the carried phase, NaN; out_0 .. out_{j-1} stay
+# within the bound.
+C_NCO_A = 2.0
+C_NCO_B = 16.0
+C_SINCOS = 6.0
+NCO_CHUNK = 1024 * 2048
+
+
+def exact_prefix(perr):
+    """Inclusive prefix sums of perr as double-double arrays (hi, lo), exact to about 2^-100 of their size.  Entries
+    on the dyadic grid int * 2^-40 (|int| < 2^30) are summed exactly in int64; the others (at most a few thousand:
+    huge values, subnormals, mixed magnitudes) are summed exactly with Fraction and added in double-double.
+    Non-finite entries give NaN from their index on."""
+    from fractions import Fraction
+    p = np.asarray(perr, np.float64)
+    fin = np.isfinite(p)
+    s = np.where(fin, p, 0.0) * 2.0 ** 40
+    grid = fin & (s == np.rint(s)) & (np.abs(s) < 2.0 ** 30)
+    ints = np.where(grid, s, 0.0).astype(np.int64)
+    hi = np.cumsum(ints).astype(np.float64) * 2.0 ** -40  # |cumsum| < 2^53: exact
+    lo = np.zeros_like(hi)
+    off = np.nonzero(fin & ~grid)[0]
+    assert len(off) <= 8192, "exact_prefix: too many off-grid entries"
+    if len(off):
+        acc = Fraction(0)
+        bounds = list(off) + [len(p)]
+        for j, (a, b) in enumerate(zip(bounds[:-1], bounds[1:])):
+            acc += Fraction(float(p[a]))
+            ah = float(acc)
+            al = float(acc - Fraction(ah))
+            h2, l2 = dd_add(hi[a:b], lo[a:b], ah, al)
+            hi[a:b], lo[a:b] = h2, l2
+    bad = np.nonzero(~fin)[0]
+    if len(bad):
+        hi[bad[0]:] = np.nan
+        lo[bad[0]:] = np.nan
+    return hi, lo
+
+
+def nco_exact(phase0, dphase, perr, start=0, prefix=None):
+    """(cos, sin) in long double of e^{j phi_k} for the outputs k = start .. start + len(perr) - 1 of a stream whose
+    phase was phase0 before its output 0; `prefix`: exact (hi, lo) prefix sums of the stream's perr at these outputs
+    (default: of perr alone, i.e. start == 0 or no earlier perr)"""
+    pre = exact_prefix(perr) if prefix is None else prefix
+    k = start + 1 + np.arange(len(perr), dtype=np.int64)
+    return _cis_ld(*phase_exact(phase0, dphase, k, pre))
+
+
+def nco_bound(phase0, S, calls=0, chunks=0):
+    return U64 * (C_NCO_A * (abs(phase0) + 2 * np.pi * (1 + calls + np.asarray(chunks))) + C_NCO_B * np.asarray(S)
+                  + C_SINCOS)
+
+
+def nco_bound_report(got, c, s, bound, nonfinite_from=None):
+    """(failures, worst index, worst ratio) of NCO outputs against (c + j s) and the per-output bound; from index
+    `nonfinite_from` on every output must be NaN (in both components)"""
+    g = np.asarray(got).astype(np.complex128)
+    n = len(g)
+    j = n if nonfinite_from is None else int(nonfinite_from)
+    err = _err_ld(g[:j], c[:j], s[:j])
+    with np.errstate(all="ignore"):
+        r = np.where(np.isfinite(err), err / np.asarray(bound)[:j], np.inf)
+    fails = []
+    bad = np.nonzero(~(r <= 1))[0]
+    if len(bad):
+        b = int(bad[0])
+        fails.append(f"NCO output {b}: |err|/bound = {r[b]:.3g} (|err| {err[b]:.3g}, bound {np.asarray(bound)[b]:.3g}); "
+                     f"{len(bad)} of {j} causal outputs outside")
+    if j < n:
+        nn = ~(np.isnan(g[j:].real) & np.isnan(g[j:].imag))
+        if nn.any():
+            fails.append(f"NCO output {j + int(np.argmax(nn))} at or after the non-finite perr[{j}] is not NaN "
+                         f"({int(nn.sum())} of {n - j})")
+    w = int(np.argmax(np.where(np.isfinite(r), r, np.inf))) if len(r) else 0
+    return fails, w, float(r[w]) if len(r) else 0.0
+
+
+# ---- f64 estimators: |est - arg S| <= asin(E / |S|) + EST_ABS
+# Frequency estimator, S = sum_{i < n-1} x_{i+1} conj(x_i):  E = C_FREQ u64 D_F sum |x_{i+1}| |x_i|, where D_F counts
+# the additions on one term's way to the result at the launch shape (P = min(ceil(n / 2048), 1184) CTAs of 256
+# threads): the product (2), the thread's run of m = ceil((n-1) / (256 P)) terms, the warp tree (5) and the CTA's 7
+# warp partials, the final CTA's ceil(P / 256) partials per thread, its warp tree and warp partials.  C_FREQ = sqrt 2
+# (each of the real and imaginary sums obeys the first-order bound D_F u64 sum |t|; the complex error is at most
+# sqrt 2 times that).  The emulation attains 0.45 of it with terms built so that one thread's additions all round the
+# same way (random-phase input: 1.3e-5).  EST_ABS = 4 ulp(pi): atan2, the reference's own rounding of arg S and the
+# roundings of -N arg / 2 pi.
+C_FREQ = np.sqrt(2.0)
+EST_ABS = 2.0 ** -49
+EST_BLOCKS = 148 * 8
+
+
+def freq_depth(n):
+    p = min(-(-max(n, 1) // 2048), EST_BLOCKS)
+    m = -(-(n - 1) // (256 * p))
+    return 2 + m + 5 + 7 + -(-p // 256) + 5 + 7
+
+
+def _dd_tree_sum(h, l):
+    """double-double sum of the pairs (h_i, l_i) by a pairwise tree"""
+    h, l = np.asarray(h, np.float64), np.asarray(l, np.float64)
+    while len(h) > 1:
+        if len(h) & 1:
+            h, l = np.append(h, 0.0), np.append(l, 0.0)
+        h, l = dd_add(h[0::2], l[0::2], h[1::2], l[1::2])
+    return (float(h[0]), float(l[0])) if len(h) else (0.0, 0.0)
+
+
+def freq_exact(x):
+    """(S as complex128 rounded from its double-double, sum |x_{i+1}| |x_i|, S as ((re hi, re lo), (im hi, im lo)))"""
+    x = np.asarray(x, np.complex128)
+    a, b = x[1:], x[:-1]
+    with np.errstate(all="ignore"):
+        p1, e1 = two_prod(a.real, b.real)
+        p2, e2 = two_prod(a.imag, b.imag)
+        p3, e3 = two_prod(a.imag, b.real)
+        p4, e4 = two_prod(a.real, b.imag)
+        re = _dd_tree_sum(np.concatenate([p1, p2]), np.concatenate([e1, e2]))
+        im = _dd_tree_sum(np.concatenate([p3, -p4]), np.concatenate([e3, -e4]))
+        T = float(np.sum(np.abs(a) * np.abs(b)))
+    return complex(re[0] + re[1], im[0] + im[1]), T, (re, im)
+
+
+def angle_dd(re, im):
+    """arg of the double-double complex number ((re hi, re lo), (im hi, im lo)), in long double"""
+    return float(np.arctan2(np.longdouble(im[0]) + np.longdouble(im[1]), np.longdouble(re[0]) + np.longdouble(re[1])))
+
+
+def est_bound_report(est, S_abs, E, arg_exact, scale=1.0, what=""):
+    """(ok, ratio, skipped): |est - arg_exact| (mod 2 pi, times `scale` for the timing estimator) within
+    scale (asin(E / |S|) + EST_ABS); skipped when E >= |S| (the estimate must still be finite)"""
+    if not (E < S_abs):
+        return bool(np.isfinite(est)), 0.0, True
+    d = abs(est - arg_exact * scale) / abs(scale)
+    d = min(d % (2 * np.pi), 2 * np.pi - d % (2 * np.pi))
+    b = np.arcsin(E / S_abs) * (1 + 1e-9) + EST_ABS
+    return d <= b, d / b, False
+
+
+# Timing estimator: S = sum_i qout_i dout_i, qout = q * qin (2ND+1 real taps), qin_m = conj(x_m) r_m, dout_i =
+# x_{i-ND} r_{i-ND}, r_m = e^{-j fl(fl(-pi m) / N)} (the reference's operation order).
+#   E = u64 (C_TIM (ntaps4 + D_T) + 2 (C_SINCOS + 2)) sum_i |dout_i| A_i,   A_i = sum_k |q_k| |qin_{i-k}|
+# ntaps4 = the FMA chain of the register window (taps padded to four), D_T the partial sums at the launch shape (the
+# product, each thread's 4 outputs per tile over its tiles, the CTA and final trees as for the frequency estimator),
+# 2 (C_SINCOS + 2) the device sincos and the products qin = conj(x) r, din = x r, which scale both factors.  C_TIM =
+# sqrt 2 as above.  This one is a worst-case first-order bound, not a calibrated one: the emulation's worst ratio on
+# noise and QPSK input is 2.7e-3 (no input was found that aligns the roundings of the 4-tap-group FMA chain).  The timing estimate is -N arg(S) / 2 pi, so its bound is (N / 2 pi) (asin(E / |S|) + EST_ABS).
+C_TIM = np.sqrt(2.0)
+
+
+def timing_depth(n, ntaps):
+    p = min(-(-max(n, 1) // 1024), EST_BLOCKS)
+    tiles = -(-(-(-n // 1024)) // p)
+    return 2 + 4 * tiles + 5 + 7 + -(-p // 256) + 5 + 7
+
+
+def timing_taps(n, d, alpha):
+    """the f64 taps the library uses: cb_qfilt_taps_f64(2 n d + 1, alpha, n), recomputed here"""
+    real_n = 2 * n * d + 1
+    dd = int(np.floor(real_n / 2.0))
+    t = np.empty(real_n)
+    for i in range(real_n):
+        tt = float(i - dd) / float(n)
+        two = 2.0 * alpha * tt
+        if abs(two) == 1.0:
+            t[i] = np.sin(np.pi * alpha * tt) / (8.0 * tt)
+        else:
+            t[i] = (alpha * np.cos(np.pi * alpha * tt)) / (np.pi * (1.0 - two * two))
+    return t
+
+
+def timing_exact(x, taps, N, D):
+    """(running S_i = sum_{i' <= i} qout_i' dout_i' as complex long double per i, running W_i = sum |dout| A, per
+    i): the exact sums of every prefix length of x, so that one call serves every n.  qout in long double by direct
+    convolution (error <= ntaps 2^-64 A_i), r from the reference's f64 argument with long double sin and cos."""
+    x = np.asarray(x, np.complex128)
+    n = len(x)
+    m = np.arange(n, dtype=np.float64)
+    arg = (-np.pi * m) / float(N)  # the f64 argument, bit for bit (pi * m first, then / N)
+    c, s = np.cos(arg.astype(np.longdouble)), np.sin(arg.astype(np.longdouble))
+    xr, xi = x.real.astype(np.longdouble), x.imag.astype(np.longdouble)
+    qin = (xr * c + xi * s) + 1j * (xr * s - xi * c)  # conj(x) r
+    din = (xr * c - xi * s) + 1j * (xr * s + xi * c)  # x r
+    t = np.asarray(taps).astype(np.longdouble)
+    qout = np.convolve(qin.astype(np.clongdouble), t)[:n]
+    A = np.convolve(np.abs(qin).astype(np.longdouble), np.abs(t))[:n]
+    nd = N * D
+    dout = np.zeros(n, np.clongdouble)
+    dout[nd:] = din[: n - nd] if nd < n else []
+    S = np.cumsum(qout * dout)
+    W = np.cumsum((np.abs(dout) * A).astype(np.float64))
+    return S, W
+
+
+def timing_E(n, ntaps, W):
+    ntaps4 = (ntaps + 3) & ~3
+    return U64 * (C_TIM * (ntaps4 + timing_depth(n, ntaps)) + 2 * (C_SINCOS + 2)) * W * (1 + 1e-6)
