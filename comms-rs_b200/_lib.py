@@ -88,6 +88,15 @@ SIGNATURES = {
     "cb_fir_get_state": (_i, [_vp, _vp, _sz]),
     "cb_fir_set_state": (_i, [_vp, _vp, _sz]),
     "cb_fir_stream": (_vp, [_vp]),
+    "cb_fir_f64_create": (_i, [_vp, _sz, _vp, _sz, _u32, _u32, _pp]),
+    "cb_fir_f64_destroy": (_i, [_vp]),
+    "cb_fir_f64_out_len": (_i, [_vp, _sz, _psz]),
+    "cb_fir_f64_run": (_i, [_vp, _vp, _sz, _vp, _sz, _psz]),
+    "cb_fir_f64_run_dev": (_i, [_vp, _vp, _sz, _vp, _sz, _psz, _vp]),
+    "cb_fir_f64_state_len": (_i, [_vp, _psz]),
+    "cb_fir_f64_get_state": (_i, [_vp, _vp, _sz]),
+    "cb_fir_f64_set_state": (_i, [_vp, _vp, _sz]),
+    "cb_fir_f64_stream": (_vp, [_vp]),
     "cb_decimate_dev": (_i, [_vp, _sz, _sz, _sz, _vp, _sz, _psz, _vp]),
     "cb_upsample_dev": (_i, [_vp, _sz, _sz, _sz, _vp, _sz, _psz, _vp]),
     "cb_decimate": (_i, [_vp, _sz, _sz, _sz, _vp, _sz, _psz]),

@@ -17,6 +17,7 @@
 #include "common.cuh"
 #include "estimator_kernels.cuh"
 #include "fft_kernels.cuh"
+#include "fir_f64_kernels.cuh"
 #include "fir_kernels.cuh"
 #include "misc_kernels.cuh"
 
@@ -881,30 +882,51 @@ int cb_copy_d2h_async(void *dst, const void *src, size_t bytes, void *stream)
 }
 
 // ============================================================================ FIR
-static size_t fir_out_len(const cb_fir *h, size_t n)
+// The helpers below serve both FIR handles (cb_fir over float2 samples, cb_fir_f64 over double2): they depend on the
+// handle's shape (interp, decim, hist_len) only.
+extern "C++" {
+template <typename Fir>
+static size_t fir_out_len(const Fir *h, size_t n)
 {
     const size_t up = n * h->interp;
     return h->decim > 1 ? ceil_div(up, (size_t)h->decim) : up;
 }
 
 // reference state (newest first, zero-stuffed domain) -> chronological input-domain history
-static int fir_state_to_hist(const cb_fir *h, const float2 *state, size_t nstate, std::vector<float2> &hist)
+template <typename Fir, typename T>
+static int fir_state_to_hist(const Fir *h, const T *state, size_t nstate, std::vector<T> &hist)
 {
-    hist.assign(h->hist_len, make_float2(0.f, 0.f));
+    hist.assign(h->hist_len, T{});
     if (!state) return CB_OK;
     const size_t L = h->interp;
     for (size_t k = 0; k < nstate; ++k) {
-        const float2 v = state[k];
+        const T v = state[k];
         if ((k + 1) % L == 0) {
             const size_t i = (k + 1) / L;  // i-th most recent input sample
             if (i <= h->hist_len) hist[h->hist_len - i] = v;
-        } else if (v.x != 0.f || v.y != 0.f) {
+        } else if (v.x != 0 || v.y != 0) {
             set_error("fir: with interp=%zu the initial state must be zero off the symbol grid (entry %zu)", L, k);
             return CB_ERR_UNSUPPORTED;
         }
     }
     return CB_OK;
 }
+
+// chronological input-domain history -> reference state (newest first, nstate entries, zero-stuffed domain)
+template <typename Fir, typename T>
+static void fir_hist_to_state(const Fir *h, const std::vector<T> &hist, T *state, size_t nstate)
+{
+    const size_t L = h->interp;
+    for (size_t k = 0; k < nstate; ++k) {
+        T v{};
+        if ((k + 1) % L == 0) {
+            const size_t i = (k + 1) / L;
+            if (i <= h->hist_len) v = hist[h->hist_len - i];
+        }
+        state[k] = v;
+    }
+}
+}  // extern "C++"
 
 int cb_fir_create(const float *taps, size_t ntaps, const float *state, size_t nstate, uint32_t decim,
                   uint32_t interp, cb_fir **out)
@@ -1499,16 +1521,7 @@ int cb_fir_get_state(cb_fir *h, float *state, size_t nstate)
     }
     std::vector<float2> hist(h->hist_len);
     CB_CUDA(cudaMemcpy(hist.data(), h->hist[h->cur], h->hist_len * sizeof(float2), cudaMemcpyDeviceToHost));
-    float2 *st = reinterpret_cast<float2 *>(state);
-    const size_t L = h->interp;
-    for (size_t k = 0; k < nstate; ++k) {
-        float2 v = make_float2(0.f, 0.f);
-        if ((k + 1) % L == 0) {
-            const size_t i = (k + 1) / L;
-            if (i <= h->hist_len) v = hist[h->hist_len - i];
-        }
-        st[k] = v;
-    }
+    fir_hist_to_state(h, hist, reinterpret_cast<float2 *>(state), nstate);
     return CB_OK;
 }
 
@@ -1524,6 +1537,218 @@ int cb_fir_set_state(cb_fir *h, const float *state, size_t nstate)
     rc = h->last.sync();
     if (rc) return rc;
     CB_CUDA(cudaMemcpy(h->hist[h->cur], hist.data(), h->hist_len * sizeof(float2), cudaMemcpyHostToDevice));
+    return CB_OK;
+}
+
+// ============================================================================ FIR over Complex<f64>
+// The same filter, state and resampling semantics as cb_fir, over double2 samples, with one direct-form kernel family
+// (fir_f64_kernels.cu) whose per-output FMA chain is fixed: no tensor-core, overlap-save or zero-copy paths.
+struct cb_fir_f64 {
+    int device;
+    cudaStream_t stream;
+    HostPipe pipe;
+    double2 *taps_dev;
+    size_t nstate;      // reference state length (zero-stuffed domain when interp > 1)
+    uint32_t k_eff;     // min(ntaps, nstate)
+    bool taps_real;
+    uint32_t decim, interp;
+    uint32_t hist_len;  // input-domain samples kept
+    double2 *hist[2];
+    int cur;
+    LastUse last;
+};
+
+int cb_fir_f64_create(const double *taps, size_t ntaps, const double *state, size_t nstate, uint32_t decim,
+                      uint32_t interp, cb_fir_f64 **out)
+{
+    CB_REQUIRE(out, CB_ERR_INVALID_ARG, "out is NULL");
+    CB_REQUIRE(taps || ntaps == 0, CB_ERR_INVALID_ARG, "taps is NULL");
+    // the kernels skip the products with stuffed zeros and padding, so a non-finite tap could not poison the outputs
+    // the way the reference's fold over the zero-stuffed stream does: reject it instead
+    for (size_t k = 0; k < 2 * ntaps; ++k)
+        CB_REQUIRE(std::isfinite(taps[k]), CB_ERR_INVALID_ARG, "fir_f64: tap %zu is not finite", k / 2);
+    int rc = ensure_device();
+    if (rc) return rc;
+    cb_fir_f64 *h = new (std::nothrow) cb_fir_f64();
+    CB_REQUIRE(h, CB_ERR_OOM, "host allocation failed");
+    h->device = g_dev;
+    h->decim = decim == 0 ? 1 : decim;
+    h->interp = interp == 0 ? 1 : interp;
+    h->nstate = state ? nstate : ntaps;  // None => zeros(len taps)  (fir_node.rs:201-210)
+    h->k_eff = (uint32_t)(ntaps < h->nstate ? ntaps : h->nstate);
+    h->taps_real = true;
+    for (size_t k = 0; k < h->k_eff; ++k)
+        if (taps[2 * k + 1] != 0.0) h->taps_real = false;
+    const size_t need_in = ceil_div(h->nstate > h->k_eff ? h->nstate : (size_t)h->k_eff, (size_t)h->interp);
+    h->hist_len = (uint32_t)(need_in > 1 ? need_in : 1);
+    h->cur = 0;
+    h->taps_dev = nullptr;
+    h->hist[0] = h->hist[1] = nullptr;
+    h->stream = nullptr;
+    std::vector<double2> hist;
+    rc = fir_state_to_hist(h, reinterpret_cast<const double2 *>(state), state ? nstate : 0, hist);
+    if (rc) {
+        delete h;
+        return rc;
+    }
+    cudaError_t e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
+    if (e == cudaSuccess && h->pipe.init(h->stream)) e = cudaErrorUnknown;
+    if (e == cudaSuccess) e = cudaMalloc(&h->taps_dev, (ntaps ? ntaps : 1) * sizeof(double2));
+    if (e == cudaSuccess && ntaps) e = cudaMemcpy(h->taps_dev, taps, ntaps * sizeof(double2), cudaMemcpyHostToDevice);
+    for (int i = 0; i < 2 && e == cudaSuccess; ++i) {
+        e = cudaMalloc(&h->hist[i], h->hist_len * sizeof(double2));
+        if (e == cudaSuccess) e = cudaMemcpy(h->hist[i], hist.data(), h->hist_len * sizeof(double2), cudaMemcpyHostToDevice);
+    }
+    if (e != cudaSuccess) {
+        cb_fir_f64_destroy(h);
+        return cuda_fail(e, "fir_f64 create", __FILE__, __LINE__);
+    }
+    *out = h;
+    return CB_OK;
+}
+
+int cb_fir_f64_destroy(cb_fir_f64 *h)
+{
+    if (!h) return CB_OK;
+    cudaSetDevice(h->device);
+    if (h->stream) cudaStreamSynchronize(h->stream);
+    h->last.destroy();
+    h->pipe.destroy();
+    if (h->taps_dev) cudaFree(h->taps_dev);
+    for (int i = 0; i < 2; ++i)
+        if (h->hist[i]) cudaFree(h->hist[i]);
+    if (h->stream) cudaStreamDestroy(h->stream);
+    delete h;
+    return CB_OK;
+}
+
+int cb_fir_f64_out_len(const cb_fir_f64 *h, size_t n_in, size_t *n_out)
+{
+    CB_REQUIRE(h && n_out, CB_ERR_INVALID_ARG, "NULL argument");
+    *n_out = fir_out_len(h, n_in);
+    return CB_OK;
+}
+
+void *cb_fir_f64_stream(cb_fir_f64 *h) { return h ? (void *)h->stream : nullptr; }
+
+static int fir64_launch(cb_fir_f64 *h, const double2 *x, size_t n, const double2 *hist_in, double2 *hist_out, double2 *y,
+                        cudaStream_t s)
+{
+    const Fir64Seg seg{x, hist_in, hist_out, y, n, fir_out_len(h, n), h->hist_len, h->k_eff, h->interp, h->decim};
+    return launch_fir_f64(seg, h->taps_dev, h->taps_real, s);
+}
+
+int cb_fir_f64_run_dev(cb_fir_f64 *h, const double *d_in, size_t n_in, double *d_out, size_t out_cap, size_t *n_out,
+                       void *stream)
+{
+    CB_REQUIRE(h, CB_ERR_INVALID_ARG, "handle is NULL");
+    const size_t no = fir_out_len(h, n_in);
+    if (n_out) *n_out = no;
+    if (n_in == 0) return CB_OK;
+    CB_REQUIRE(d_in && d_out, CB_ERR_INVALID_ARG, "NULL data pointer");
+    CB_REQUIRE(((reinterpret_cast<uintptr_t>(d_in) | reinterpret_cast<uintptr_t>(d_out)) & 15) == 0, CB_ERR_INVALID_ARG,
+               "fir_f64: d_in and d_out must be 16-byte aligned");  // read and written as double2
+    CB_REQUIRE(out_cap >= no, CB_ERR_SIZE, "fir_f64: out_cap %zu < %zu outputs", out_cap, no);
+    CB_NO_ALIAS(d_in, n_in * sizeof(double2), d_out, no * sizeof(double2), "fir_f64");
+    CB_CUDA(cudaSetDevice(h->device));
+    cudaStream_t s = pick_stream(stream, h->stream);
+    int rc = h->last.begin(s);
+    if (rc) return rc;
+    rc = fir64_launch(h, reinterpret_cast<const double2 *>(d_in), n_in, h->hist[h->cur], h->hist[h->cur ^ 1],
+                      reinterpret_cast<double2 *>(d_out), s);
+    if (rc) return rc;
+    h->cur ^= 1;
+    return h->last.end(s);
+}
+
+// Host Vec in / Vec out: chunks of HOST_CHUNK samples pipelined over the handle's two lanes (H2D, filter, D2H); each
+// chunk after the first re-sends the previous chunk's last hist_len samples as its history.
+int cb_fir_f64_run(cb_fir_f64 *h, const double *in, size_t n_in, double *out, size_t out_cap, size_t *n_out)
+{
+    CB_REQUIRE(h, CB_ERR_INVALID_ARG, "handle is NULL");
+    const size_t no = fir_out_len(h, n_in);
+    if (n_out) *n_out = no;
+    if (n_in == 0) return CB_OK;
+    CB_REQUIRE(in && out, CB_ERR_INVALID_ARG, "NULL data pointer");
+    CB_REQUIRE(out_cap >= no, CB_ERR_SIZE, "fir_f64: out_cap %zu < %zu outputs", out_cap, no);
+    CB_CUDA(cudaSetDevice(h->device));
+    const double2 *hin = reinterpret_cast<const double2 *>(in);
+    double2 *hout = reinterpret_cast<double2 *>(out);
+    const size_t H = h->hist_len;
+    size_t chunk = HOST_CHUNK / h->decim * h->decim;  // chunk starts keep the decimation grid
+    if (chunk < 4 * H || n_in <= chunk) chunk = n_in;
+    const size_t chunk_out = fir_out_len(h, chunk);
+    int rc = h->last.sync();  // a *_run_dev on a caller's stream may still be using the carried state
+    if (rc) return rc;
+    rc = h->pipe.reserve((chunk + H) * sizeof(double2), chunk_out * sizeof(double2));
+    if (rc) return rc;
+    rc = h->pipe.begin_call(in, n_in * sizeof(double2), (chunk + H) * sizeof(double2), out, no * sizeof(double2),
+                            chunk_out * sizeof(double2));
+    if (rc) return rc;
+    size_t done = 0, out_done = 0;
+    for (int i = 0; done < n_in; ++i) {
+        const int l = i & 1;
+        const size_t n = n_in - done < chunk ? n_in - done : chunk;
+        const bool last = done + n == n_in;
+        cudaStream_t s = h->pipe.lane[l];
+        double2 *slot = reinterpret_cast<double2 *>(h->pipe.in[l]);
+        const double2 *hist_in;
+        if (done == 0) {
+            hist_in = h->hist[h->cur];
+            rc = h->pipe.h2d(l, slot + H, hin, n * sizeof(double2));
+        } else {
+            hist_in = slot;
+            rc = h->pipe.h2d(l, slot, hin + done - H, (n + H) * sizeof(double2));
+        }
+        if (rc) return rc;
+        double2 *y = reinterpret_cast<double2 *>(h->pipe.out[l]);
+        rc = fir64_launch(h, slot + H, n, hist_in, last ? h->hist[h->cur ^ 1] : nullptr, y, s);
+        if (rc) return rc;
+        const size_t m = fir_out_len(h, n);
+        rc = h->pipe.d2h(l, hout + out_done, y, m * sizeof(double2));
+        if (rc) return rc;
+        done += n;
+        out_done += m;
+    }
+    rc = h->pipe.sync();
+    if (rc) return rc;
+    h->cur ^= 1;
+    return CB_OK;
+}
+
+int cb_fir_f64_state_len(const cb_fir_f64 *h, size_t *nstate)
+{
+    CB_REQUIRE(h && nstate, CB_ERR_INVALID_ARG, "NULL argument");
+    *nstate = h->nstate;
+    return CB_OK;
+}
+
+int cb_fir_f64_get_state(cb_fir_f64 *h, double *state, size_t nstate)
+{
+    CB_REQUIRE(h && (state || nstate == 0), CB_ERR_INVALID_ARG, "NULL argument");
+    CB_REQUIRE(nstate == h->nstate, CB_ERR_SIZE, "fir_f64: state length %zu != %zu", nstate, h->nstate);
+    CB_CUDA(cudaSetDevice(h->device));
+    CB_CUDA(cudaStreamSynchronize(h->stream));
+    int rc = h->last.sync();
+    if (rc) return rc;
+    std::vector<double2> hist(h->hist_len);
+    CB_CUDA(cudaMemcpy(hist.data(), h->hist[h->cur], h->hist_len * sizeof(double2), cudaMemcpyDeviceToHost));
+    fir_hist_to_state(h, hist, reinterpret_cast<double2 *>(state), nstate);
+    return CB_OK;
+}
+
+int cb_fir_f64_set_state(cb_fir_f64 *h, const double *state, size_t nstate)
+{
+    CB_REQUIRE(h && state, CB_ERR_INVALID_ARG, "NULL argument");
+    CB_REQUIRE(nstate == h->nstate, CB_ERR_SIZE, "fir_f64: state length %zu != %zu", nstate, h->nstate);
+    CB_CUDA(cudaSetDevice(h->device));
+    std::vector<double2> hist;
+    int rc = fir_state_to_hist(h, reinterpret_cast<const double2 *>(state), nstate, hist);
+    if (rc) return rc;
+    CB_CUDA(cudaStreamSynchronize(h->stream));
+    rc = h->last.sync();
+    if (rc) return rc;
+    CB_CUDA(cudaMemcpy(h->hist[h->cur], hist.data(), h->hist_len * sizeof(double2), cudaMemcpyHostToDevice));
     return CB_OK;
 }
 

@@ -283,6 +283,54 @@ struct NcoBatchNode : Node1<NcoBatchNode, std::vector<double>, std::vector<c64>>
     }
 };
 
+// The FIR over Complex<f64> (cb_fir_f64): same constructor arguments and run() meaning as the f32 nodes
+class FirF64Handle {
+protected:
+    cb_fir_f64 *h_ = nullptr;
+public:
+    FirF64Handle(const std::vector<c64> &taps, const std::vector<c64> *state, uint32_t decim, uint32_t interp)
+    {
+        int st = cb_fir_f64_create(reinterpret_cast<const double *>(taps.data()), taps.size(),
+                                   state ? reinterpret_cast<const double *>(state->data()) : nullptr,
+                                   state ? state->size() : 0, decim, interp, &h_);
+        if (st) throw std::runtime_error(std::string("cb_fir_f64_create: ") + cb_last_error());
+    }
+    FirF64Handle(const FirF64Handle &) = delete;
+    ~FirF64Handle() { cb_fir_f64_destroy(h_); }
+    Result<std::vector<c64>> filter(const c64 *in, size_t n)
+    {
+        size_t no = 0;
+        cb_fir_f64_out_len(h_, n, &no);
+        std::vector<c64> out(no);
+        int st = cb_fir_f64_run(h_, reinterpret_cast<const double *>(in), n, reinterpret_cast<double *>(out.data()), no, &no);
+        if (st) return Result<std::vector<c64>>::Err(map_status(st));
+        out.resize(no);
+        return Result<std::vector<c64>>::Ok(std::move(out));
+    }
+    std::vector<c64> state()
+    {
+        size_t n = 0;
+        cb_fir_f64_state_len(h_, &n);
+        std::vector<c64> s(n);
+        cb_fir_f64_get_state(h_, reinterpret_cast<double *>(s.data()), n);
+        return s;
+    }
+};
+
+// BatchFirNode<Complex<f64>>::new(taps, state) / run(&[Complex<f64>])   src/filter/fir_node.rs:193-220
+struct BatchFirNodeF64 : Node1<BatchFirNodeF64, std::vector<c64>, std::vector<c64>>, FirF64Handle {
+    BatchFirNodeF64(const std::vector<c64> &taps, const std::vector<c64> *state = nullptr, uint32_t decim = 1,
+                    uint32_t interp = 1)
+        : FirF64Handle(taps, state, decim, interp) {}
+    Result<std::vector<c64>> run(const std::vector<c64> &in) { return filter(in.data(), in.size()); }
+};
+
+// PulseNode<f64>::new(taps, sam_per_sym) / run(&Complex<f64>) -> Vec   src/pulse.rs:71-92
+struct PulseNodeF64 : Node1<PulseNodeF64, c64, std::vector<c64>>, FirF64Handle {
+    PulseNodeF64(const std::vector<c64> &taps, size_t sam_per_sym) : FirF64Handle(taps, nullptr, 1, (uint32_t)sam_per_sym) {}
+    Result<std::vector<c64>> run(const c64 &sym) { return filter(&sym, 1); }
+};
+
 // FFTBatchNode::new(fft_size, ifft) / run(&[Complex<T>])      src/fft/fft_node.rs:65-83
 struct FFTBatchNode : Node1<FFTBatchNode, std::vector<c32>, std::vector<c32>> {
     cb_fft *h_ = nullptr;

@@ -176,6 +176,81 @@ class PulseNode(BatchFirNode):
         self.sam_per_sym = sam_per_sym
 
 
+def _c128(a) -> np.ndarray:
+    return np.ascontiguousarray(np.asarray(a, dtype=np.complex128))
+
+
+class BatchFirNodeF64(_Handle):
+    """BatchFirNode<Complex<f64>> (src/filter/fir_node.rs:193-211) over complex128, with the neighbouring
+    Upsample/Decimate nodes optionally fused (interp / decim).  Every output is the fixed FMA chain stated in
+    include/comms_b200.h (cb_fir_f64), so call splits and host/device entries give the same bits."""
+
+    _destroy = "cb_fir_f64_destroy"
+
+    def __init__(self, taps, state=None, decim: int = 1, interp: int = 1):
+        super().__init__()
+        t = _c128(taps)
+        s = None if state is None else _c128(state)
+        check(_lib.load().cb_fir_f64_create(_ptr(t), len(t), None if s is None else _ptr(s), 0 if s is None else len(s),
+                                            decim, interp, C.byref(self._h)))
+
+    def out_len(self, n_in: int) -> int:
+        m = _sz()
+        check(_lib.load().cb_fir_f64_out_len(self._h, n_in, C.byref(m)))
+        return m.value
+
+    def run(self, samples) -> np.ndarray:
+        x = _c128(samples)
+        out = np.empty(self.out_len(len(x)), dtype=np.complex128)
+        m = _sz()
+        try:
+            check(_lib.load().cb_fir_f64_run(self._h, _ptr(x), len(x), _ptr(out), len(out), C.byref(m)))
+        except CbError as e:
+            raise node_error(e) from e
+        return out[: m.value]
+
+    def run_dev(self, d_in: int, n_in: int, d_out: int, out_cap: int, stream: int = 0) -> int:
+        """n_in complex f64 in, out_cap of room; device pointers, 16-byte aligned.  Returns the number of outputs."""
+        m = _sz()
+        check(_lib.load().cb_fir_f64_run_dev(self._h, d_in, n_in, d_out, out_cap, C.byref(m), stream))
+        return m.value
+
+    @property
+    def state(self) -> np.ndarray:
+        n = _sz()
+        check(_lib.load().cb_fir_f64_state_len(self._h, C.byref(n)))
+        st = np.empty(n.value, dtype=np.complex128)
+        check(_lib.load().cb_fir_f64_get_state(self._h, _ptr(st), n.value))
+        return st
+
+    @state.setter
+    def state(self, value):
+        s = _c128(value)
+        check(_lib.load().cb_fir_f64_set_state(self._h, _ptr(s), len(s)))
+
+    @property
+    def stream(self) -> int:
+        return _lib.load().cb_fir_f64_stream(self._h) or 0
+
+
+class FirNodeF64(BatchFirNodeF64):
+    """FirNode<Complex<f64>> (src/filter/fir_node.rs:43-114): one sample per run()."""
+
+    def run(self, sample) -> np.complex128:  # type: ignore[override]
+        return super().run(np.asarray([sample], dtype=np.complex128))[0]
+
+
+class PulseNodeF64(BatchFirNodeF64):
+    """PulseNode<f64>::new(taps, sam_per_sym) (src/pulse.rs:71-80): one symbol in, `sam_per_sym` samples out;
+    run() also accepts a batch of symbols."""
+
+    def __init__(self, taps, sam_per_sym: int):
+        if sam_per_sym < 1:
+            raise NodeError(NodeError.DataError, "sam_per_sym must be >= 1")
+        super().__init__(taps, None, decim=1, interp=sam_per_sym)
+        self.sam_per_sym = sam_per_sym
+
+
 class _Resample:
     _fn = ""
 

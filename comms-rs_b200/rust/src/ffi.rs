@@ -3,7 +3,7 @@
 use std::os::raw::{c_char, c_double, c_float, c_int, c_uint, c_void};
 
 macro_rules! opaque { ($($n:ident),*) => { $(#[repr(C)] pub struct $n { _p: [u8; 0] })* } }
-opaque!(cb_stream, cb_buf, cb_fir, cb_mixer, cb_fft, cb_fm, cb_chain, cb_comm, cb_timing, cb_nco);
+opaque!(cb_stream, cb_buf, cb_fir, cb_mixer, cb_fft, cb_fm, cb_chain, cb_comm, cb_timing, cb_nco, cb_fir_f64);
 
 pub const CB_OK: c_int = 0;
 pub const CB_ERR_INVALID_ARG: c_int = 1;
@@ -48,6 +48,19 @@ extern "C" {
     pub fn cb_fir_get_state(h: *mut cb_fir, state: *mut c_float, nstate: usize) -> c_int;
     pub fn cb_fir_set_state(h: *mut cb_fir, state: *const c_float, nstate: usize) -> c_int;
     pub fn cb_fir_stream(h: *mut cb_fir) -> *mut c_void;
+
+    pub fn cb_fir_f64_create(taps: *const f64, ntaps: usize, state: *const f64, nstate: usize,
+                             decim: u32, interp: u32, out: *mut *mut cb_fir_f64) -> c_int;
+    pub fn cb_fir_f64_destroy(h: *mut cb_fir_f64) -> c_int;
+    pub fn cb_fir_f64_out_len(h: *const cb_fir_f64, n_in: usize, n_out: *mut usize) -> c_int;
+    pub fn cb_fir_f64_run(h: *mut cb_fir_f64, input: *const f64, n_in: usize, out: *mut f64, out_cap: usize,
+                          n_out: *mut usize) -> c_int;
+    pub fn cb_fir_f64_run_dev(h: *mut cb_fir_f64, d_in: *const f64, n_in: usize, d_out: *mut f64, out_cap: usize,
+                              n_out: *mut usize, stream: *mut c_void) -> c_int;
+    pub fn cb_fir_f64_state_len(h: *const cb_fir_f64, nstate: *mut usize) -> c_int;
+    pub fn cb_fir_f64_get_state(h: *mut cb_fir_f64, state: *mut f64, nstate: usize) -> c_int;
+    pub fn cb_fir_f64_set_state(h: *mut cb_fir_f64, state: *const f64, nstate: usize) -> c_int;
+    pub fn cb_fir_f64_stream(h: *mut cb_fir_f64) -> *mut c_void;
 
     pub fn cb_decimate(input: *const c_void, n: usize, elem_bytes: usize, rate: usize, out: *mut c_void,
                        out_cap: usize, n_out: *mut usize) -> c_int;

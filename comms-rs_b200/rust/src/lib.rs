@@ -151,6 +151,64 @@ impl GpuBatchPulseNode {
     pub fn run(&mut self, input: &[C32]) -> Result<Vec<C32>, NodeError> { fir_run(&self.fir, input) }
 }
 
+type C64 = Complex<f64>;
+handle!(FirF64, ffi::cb_fir_f64, ffi::cb_fir_f64_destroy);
+
+fn as_f64(v: &[C64]) -> *const f64 { v.as_ptr() as *const f64 } // Complex<f64> is #[repr(C)] {re, im}
+
+fn fir_f64_new(taps: &[C64], state: Option<&[C64]>, decim: u32, interp: u32) -> FirF64 {
+    let mut h = ptr::null_mut();
+    let (sp, sn) = state.map_or((ptr::null(), 0), |s| (as_f64(s), s.len()));
+    let st = unsafe { ffi::cb_fir_f64_create(as_f64(taps), taps.len(), sp, sn, decim, interp, &mut h) };
+    assert_eq!(st, ffi::CB_OK, "cb_fir_f64_create failed (non-finite tap, or no CUDA device?)");
+    FirF64(h)
+}
+
+fn fir_f64_run(h: &FirF64, input: &[C64]) -> Result<Vec<C64>, NodeError> {
+    let mut n_out = 0usize;
+    check(unsafe { ffi::cb_fir_f64_out_len(h.0, input.len(), &mut n_out) })?;
+    let mut out: Vec<C64> = Vec::with_capacity(n_out);
+    check(unsafe { ffi::cb_fir_f64_run(h.0, as_f64(input), input.len(), out.as_mut_ptr() as *mut f64, n_out, &mut n_out) })?;
+    unsafe { out.set_len(n_out) };
+    Ok(out)
+}
+
+/// Drop-in for `BatchFirNode<f64>` (src/filter/fir_node.rs:146-221) over `Complex<f64>`.
+#[derive(Node)]
+#[pass_by_ref]
+pub struct GpuBatchFirNodeF64 {
+    pub input: NodeReceiver<Vec<C64>>,
+    fir: FirF64,
+    pub output: NodeSender<Vec<C64>>,
+}
+
+impl GpuBatchFirNodeF64 {
+    pub fn new(taps: Vec<C64>, state: Option<Vec<C64>>) -> Self {
+        GpuBatchFirNodeF64 { fir: fir_f64_new(&taps, state.as_deref(), 1, 1), input: Default::default(), output: Default::default() }
+    }
+    /// FIR with the neighbouring `UpsampleNode(interp)` / `DecimateNode(decim)` fused.
+    pub fn with_resampling(taps: Vec<C64>, state: Option<Vec<C64>>, decim: u32, interp: u32) -> Self {
+        GpuBatchFirNodeF64 { fir: fir_f64_new(&taps, state.as_deref(), decim, interp), input: Default::default(), output: Default::default() }
+    }
+    pub fn run(&mut self, input: &[C64]) -> Result<Vec<C64>, NodeError> { fir_f64_run(&self.fir, input) }
+}
+
+/// Drop-in for `PulseNode<f64>` (src/pulse.rs:36-92): one symbol in, `sam_per_sym` samples out.
+#[derive(Node)]
+#[pass_by_ref]
+pub struct GpuPulseNodeF64 {
+    pub input: NodeReceiver<C64>,
+    fir: FirF64,
+    pub output: NodeSender<Vec<C64>>,
+}
+
+impl GpuPulseNodeF64 {
+    pub fn new(taps: Vec<C64>, sam_per_sym: usize) -> Self {
+        GpuPulseNodeF64 { fir: fir_f64_new(&taps, None, 1, sam_per_sym as u32), input: Default::default(), output: Default::default() }
+    }
+    pub fn run(&mut self, input: &C64) -> Result<Vec<C64>, NodeError> { fir_f64_run(&self.fir, std::slice::from_ref(input)) }
+}
+
 /// Drop-in for `DecimateNode<T>` (src/util/resample_node.rs:18-65) for plain-old-data `T`.
 #[derive(Node)]
 #[pass_by_ref]

@@ -201,6 +201,43 @@ CB_API int cb_fir_get_state(cb_fir *h, float *state, size_t nstate);
 CB_API int cb_fir_set_state(cb_fir *h, const float *state, size_t nstate);
 CB_API void *cb_fir_stream(cb_fir *h);
 
+/* ------------------------------------------------------------------ FIR over Complex<f64>
+ * batch_fir over Complex<f64> (src/filter/fir.rs:87-102; BatchFirNode<Complex<f64>>, PulseNode<f64>): cb_fir entry for
+ * entry, with 2*n interleaved doubles wherever cb_fir has floats.  Same semantics: the zip truncation to
+ * min(ntaps, nstate) taps, state NULL = zeros of length ntaps, the state carried across calls newest first, decim /
+ * interp 0 or 1 = pass-through, the decimation phase reset on every call, the interp state in the zero-stuffed domain
+ * (an off-grid non-zero initial state gives CB_ERR_UNSUPPORTED), and the same lengths, CB_ERR_SIZE, overlap check and
+ * ordering across streams.  Two differences:
+ *   - d_in and d_out of cb_fir_f64_run_dev must be 16-byte aligned (read and written as pairs of doubles); other
+ *     pointers return CB_ERR_INVALID_ARG before any launch.
+ *   - a non-finite tap returns CB_ERR_INVALID_ARG from cb_fir_f64_create.  (The reference would multiply it by the
+ *     stuffed zeros and padding and make every output NaN; the kernels never form those products.)
+ * Operation order.  Every output is two FMA chains, real and imaginary part, each starting from +0 and running over
+ * the output's taps in ascending tap index; only taps that meet a real input sample enter a chain (never a stuffed
+ * zero, a padding tap or history older than the state):
+ *   complex taps:  re = fma(h.re, x.re, re); re = fma(-h.im, x.im, re); im = fma(h.re, x.im, im); im = fma(h.im, x.re, im)
+ *   all-real taps: re = fma(h.re, x.re, re); im = fma(h.re, x.im, im)
+ * The order does not depend on tiles, call splits, host chunks, decim or the kernel, so any split of a stream into
+ * calls gives bit-identical outputs, cb_fir_f64_run and cb_fir_f64_run_dev give bit-identical outputs, and the
+ * decimating filter's outputs are every D-th output of the plain filter of the same call, bit for bit.
+ * Accuracy.  With K_n the taps in output n's chain, u = 2^-53 and A_n = sum over those taps of |h_k| |x_{n-k}|:
+ *   |y_n - y_exact| <= 3 K_n u A_n + K_n 2^-1072     (A_n = 0 gives exactly 0)
+ * (gamma_{2K} on each chain: each term |h.re x.re| + |h.im x.im| <= |h| |x|, and sqrt(2) * 2 < 3.)
+ * Output n is non-finite (in either part) exactly when one of the input samples its taps reach is non-finite; no
+ * other output changes.  (tests/test_gpu_fir_f64.py checks every output bit for bit against a CPU emulation.) */
+typedef struct cb_fir_f64 cb_fir_f64;
+CB_API int cb_fir_f64_create(const double *taps, size_t ntaps, const double *state, size_t nstate, uint32_t decim,
+                             uint32_t interp, cb_fir_f64 **out);
+CB_API int cb_fir_f64_destroy(cb_fir_f64 *h);
+CB_API int cb_fir_f64_out_len(const cb_fir_f64 *h, size_t n_in, size_t *n_out);
+CB_API int cb_fir_f64_run(cb_fir_f64 *h, const double *in, size_t n_in, double *out, size_t out_cap, size_t *n_out);
+CB_API int cb_fir_f64_run_dev(cb_fir_f64 *h, const double *d_in, size_t n_in, double *d_out, size_t out_cap,
+                              size_t *n_out, void *stream);
+CB_API int cb_fir_f64_state_len(const cb_fir_f64 *h, size_t *nstate);
+CB_API int cb_fir_f64_get_state(cb_fir_f64 *h, double *state, size_t nstate);
+CB_API int cb_fir_f64_set_state(cb_fir_f64 *h, const double *state, size_t nstate);
+CB_API void *cb_fir_f64_stream(cb_fir_f64 *h);
+
 /* ------------------------------------------------------------------ resample
  * Stand-alone DecimateNode::decimate / UpsampleNode::upsample
  * (src/util/resample_node.rs:53-65, :120-131) for graphs that keep them as
