@@ -5,7 +5,7 @@ reference's node structs used by tests and bench.  No CPU fallback exists.
 """
 from . import _lib
 from ._lib import CbError, NodeError, load
-from .nodes import (BatchFirNode, BatchFirNodeF64, FirNodeF64, PulseNodeF64, ChainBank, DecimateNode, FFTBatchNode, FFTSampleNode, FirNode, FMDemodNode,
+from .nodes import (BatchFirNode, BatchFirNodeF64, FirNodeF64, PulseNodeF64, ChainBank, DecimateNode, FFTBatchNode, FFTBatchNodeF64, FFTSampleNode, FFTSampleNodeF64, FirNode, FMDemodNode,
                     MixerNode, NcoNode, PulseNode, UpsampleNode, bits_to_symbols_dev, complex_real_dev, convert_i16_dev, convert_u8_dev,
                     prn_bits, real_to_complex_dev,
                     quantize_i16_dev,

@@ -97,6 +97,11 @@ SIGNATURES = {
     "cb_fir_f64_get_state": (_i, [_vp, _vp, _sz]),
     "cb_fir_f64_set_state": (_i, [_vp, _vp, _sz]),
     "cb_fir_f64_stream": (_vp, [_vp]),
+    "cb_fft_f64_create": (_i, [_sz, _i, _pp]),
+    "cb_fft_f64_destroy": (_i, [_vp]),
+    "cb_fft_f64_size": (_i, [_vp, _psz, C.POINTER(_i)]),
+    "cb_fft_f64_run": (_i, [_vp, _vp, _sz, _vp]),
+    "cb_fft_f64_run_dev": (_i, [_vp, _vp, _sz, _vp, _vp]),
     "cb_decimate_dev": (_i, [_vp, _sz, _sz, _sz, _vp, _sz, _psz, _vp]),
     "cb_upsample_dev": (_i, [_vp, _sz, _sz, _sz, _vp, _sz, _psz, _vp]),
     "cb_decimate": (_i, [_vp, _sz, _sz, _sz, _vp, _sz, _psz]),

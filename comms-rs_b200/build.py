@@ -8,7 +8,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libcomms_b200.so")
-SOURCES = ["api.cu", "comm.cu", "fir_kernels.cu", "fir_tc_kernel.cu", "fir_ptc_kernel.cu", "fir_real_kernel.cu", "fft_kernels.cu", "fft_cluster_kernel.cu", "fft_cpipe_kernel.cu", "fft_rows_kernel.cu", "fft_big_kernel.cu", "chain_kernels.cu", "chain_tc_kernel.cu", "misc_kernels.cu", "estimator_kernels.cu", "nco_kernel.cu", "fir_f64_kernels.cu"]
+SOURCES = ["api.cu", "comm.cu", "fir_kernels.cu", "fir_tc_kernel.cu", "fir_ptc_kernel.cu", "fir_real_kernel.cu", "fft_kernels.cu", "fft_cluster_kernel.cu", "fft_cpipe_kernel.cu", "fft_rows_kernel.cu", "fft_big_kernel.cu", "chain_kernels.cu", "chain_tc_kernel.cu", "misc_kernels.cu", "estimator_kernels.cu", "nco_kernel.cu", "fir_f64_kernels.cu", "fft_f64_kernels.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

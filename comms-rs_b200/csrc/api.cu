@@ -17,6 +17,8 @@
 #include "common.cuh"
 #include "estimator_kernels.cuh"
 #include "fft_kernels.cuh"
+#include "fft64_core.cuh"
+#include "fft_f64_kernels.cuh"
 #include "fir_f64_kernels.cuh"
 #include "fir_kernels.cuh"
 #include "misc_kernels.cuh"
@@ -2383,6 +2385,222 @@ int cb_fft_run_iq16(cb_fft *h, const int16_t *in, size_t n_in, float in_scale, f
         rc = fft_exec_iq16(h, reinterpret_cast<const int16_t *>(h->pipe.in[l]), in_scale, dout, m / N, l, s);
         if (rc) return rc;
         rc = h->pipe.d2h(l, hout + done, dout, m * sizeof(float2));
+        if (rc) return rc;
+        done += m;
+    }
+    return h->pipe.sync();
+}
+
+// ============================================================================ FFT over Complex<f64>
+// The plan picks its path from the size alone (fft64_core.cuh, "plan shape"); every rounding is in the host/device
+// functions of fft64_core.cuh, so the CPU emulation reproduces the bits.
+enum { F64_DIRECT = 0, F64_FRAMES = 1, F64_TWOSTEP = 2, F64_CHIRPZ = 3 };
+
+struct cb_fft_f64 {
+    int device;
+    cudaStream_t stream;
+    HostPipe pipe;
+    size_t n;
+    int inverse;
+    int kind;
+    unsigned log2n;               // powers of two: log2 n; chirp-z: log2 m
+    size_t m;                     // chirp-z: the padded power of two
+    double2 *tw;                  // n-entry twiddle table of the plan's sign (chirp-z: m entries, forward)
+    double2 *tw_inv;              // chirp-z: m entries, inverse
+    double2 *chirp, *bspec;       // chirp-z: n chirp values, m spectrum values (1/m folded in)
+    double2 *scratch, *bufa, *bufb;  // two-step intermediate / chirp-z work buffers, `group` frames each
+    size_t group;
+    LastUse last;
+};
+
+static int f64_upload(const std::vector<f64fft::z64> &v, double2 **dev)
+{
+    CB_CUDA(cudaMalloc(dev, v.size() * sizeof(double2)));
+    CB_CUDA(cudaMemcpy(*dev, v.data(), v.size() * sizeof(double2), cudaMemcpyHostToDevice));
+    return CB_OK;
+}
+
+// Transforms of 2^L points (L >= 3): one frame-kernel launch up to 2^FRAME_MAX_LOG2, else two launches per group of
+// frames through the scratch: N1-point transforms down the columns (stride N2) with the inter-step twiddle tw[k1 n2]
+// applied on the way out, then N2-point transforms of the rows, stored transposed (X[k1 + N1 k2]).
+static int f64_pow2(unsigned L, const double2 *tw, int inverse, const double2 *in, double2 *out, size_t frames,
+                    double2 *scratch, size_t group, cudaStream_t s)
+{
+    const size_t N = (size_t)1 << L;
+    if (L <= f64fft::FRAME_MAX_LOG2) {
+        const Fft64Cols a{in, out, tw, nullptr, 1, N, 0, 1, N, 0, 1, L, (unsigned)frames, 1};
+        return launch_fft64_cols(a, inverse, s);
+    }
+    const unsigned L1 = L / 2, L2 = L - L1;
+    const size_t N1 = (size_t)1 << L1, N2 = (size_t)1 << L2;
+    for (size_t done = 0; done < frames;) {
+        const size_t g = frames - done < group ? frames - done : group;
+        const Fft64Cols a{in + done * N, scratch, tw, tw, N2, 1, N, 1, N1, N, (unsigned)N2, L1, (unsigned)N2, g};
+        int rc = launch_fft64_cols(a, inverse, s);
+        if (rc) return rc;
+        const Fft64Cols b{scratch, out + done * N, tw, nullptr, N1, 1, N, N1, 1, N, (unsigned)N1, L2, (unsigned)N1, g};
+        rc = launch_fft64_cols(b, inverse, s);
+        if (rc) return rc;
+        done += g;
+    }
+    return CB_OK;
+}
+
+static int f64_exec(cb_fft_f64 *h, const double2 *in, double2 *out, size_t frames, cudaStream_t s)
+{
+    const unsigned N = (unsigned)h->n;
+    if (h->kind == F64_DIRECT) return launch_fft64_direct(in, out, h->tw, N, frames, s);
+    if (h->kind != F64_CHIRPZ) return f64_pow2(h->log2n, h->tw, h->inverse, in, out, frames, h->scratch, h->group, s);
+    const unsigned M = (unsigned)h->m;
+    for (size_t done = 0; done < frames;) {
+        const size_t g = frames - done < h->group ? frames - done : h->group;
+        int rc = launch_fft64_chirp_pre(in + done * N, h->chirp, h->bufa, N, M, g, s);
+        if (!rc) rc = f64_pow2(h->log2n, h->tw, 0, h->bufa, h->bufb, g, h->scratch, g, s);
+        if (!rc) rc = launch_fft64_chirp_mul(h->bufb, h->bspec, M, g, s);
+        if (!rc) rc = f64_pow2(h->log2n, h->tw_inv, 1, h->bufb, h->bufa, g, h->scratch, g, s);
+        if (!rc) rc = launch_fft64_chirp_post(h->bufa, h->chirp, out + done * N, N, M, g, s);
+        if (rc) return rc;
+        done += g;
+    }
+    return CB_OK;
+}
+
+int cb_fft_f64_create(size_t fft_size, int inverse, cb_fft_f64 **out)
+{
+    using namespace f64fft;
+    CB_REQUIRE(out, CB_ERR_INVALID_ARG, "out is NULL");
+    CB_REQUIRE(fft_size >= 1, CB_ERR_INVALID_ARG, "fft_f64: size must be >= 1");
+    const bool pow2 = (fft_size & (fft_size - 1)) == 0;
+    CB_REQUIRE(fft_size <= ((size_t)1 << (pow2 ? 20 : 19)), CB_ERR_UNSUPPORTED, "fft_f64: size %zu is not provided",
+               fft_size);
+    int rc = ensure_device();
+    if (rc) return rc;
+    cb_fft_f64 *h = new (std::nothrow) cb_fft_f64();
+    CB_REQUIRE(h, CB_ERR_OOM, "host allocation failed");
+    h->device = g_dev;
+    h->n = fft_size;
+    h->inverse = inverse ? 1 : 0;
+    unsigned L = 0;
+    while (((size_t)1 << L) < fft_size) ++L;
+    h->log2n = L;
+    if (pow2 && L >= 3) h->kind = L <= FRAME_MAX_LOG2 ? F64_FRAMES : F64_TWOSTEP;
+    else if (pow2 || fft_size <= DIRECT_MAX) h->kind = F64_DIRECT;
+    else {
+        h->kind = F64_CHIRPZ;
+        h->m = 8;
+        while (h->m < 2 * fft_size - 1) h->m <<= 1;
+        h->log2n = 0;
+        while (((size_t)1 << h->log2n) < h->m) ++h->log2n;
+    }
+    // two-step and chirp-z work in groups of frames whose buffers take 64 MiB each
+    const size_t span = h->kind == F64_CHIRPZ ? h->m : fft_size;
+    h->group = ((size_t)64 << 20) / (span * sizeof(double2));
+    if (h->group < 1) h->group = 1;
+    cudaError_t e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
+    if (e != cudaSuccess) {
+        h->stream = nullptr;
+        cb_fft_f64_destroy(h);
+        return cuda_fail(e, "cudaStreamCreateWithFlags", __FILE__, __LINE__);
+    }
+    rc = h->pipe.init(h->stream);
+    if (!rc && h->kind != F64_CHIRPZ) rc = f64_upload(twiddle_table(fft_size, h->inverse), &h->tw);
+    if (!rc && h->kind == F64_CHIRPZ) {
+        std::vector<z64> chirp, bspec;
+        chirp_tables(fft_size, h->m, h->inverse, chirp, bspec);
+        rc = f64_upload(chirp, &h->chirp);
+        if (!rc) rc = f64_upload(bspec, &h->bspec);
+        if (!rc) rc = f64_upload(twiddle_table(h->m, 0), &h->tw);
+        if (!rc) rc = f64_upload(twiddle_table(h->m, 1), &h->tw_inv);
+        if (!rc && cudaMalloc(&h->bufa, h->group * h->m * sizeof(double2)) != cudaSuccess) rc = CB_ERR_OOM;
+        if (!rc && cudaMalloc(&h->bufb, h->group * h->m * sizeof(double2)) != cudaSuccess) rc = CB_ERR_OOM;
+    }
+    if (!rc && h->log2n > FRAME_MAX_LOG2 && cudaMalloc(&h->scratch, h->group * span * sizeof(double2)) != cudaSuccess)
+        rc = CB_ERR_OOM;
+    if (rc) {
+        if (rc == CB_ERR_OOM) {
+            cudaGetLastError();
+            set_error("fft_f64: work buffer allocation failed");
+        }
+        cb_fft_f64_destroy(h);
+        return rc;
+    }
+    *out = h;
+    return CB_OK;
+}
+
+int cb_fft_f64_destroy(cb_fft_f64 *h)
+{
+    if (!h) return CB_OK;
+    cudaSetDevice(h->device);
+    if (h->stream) cudaStreamSynchronize(h->stream);
+    h->last.destroy();
+    h->pipe.destroy();
+    for (double2 *p : {h->tw, h->tw_inv, h->chirp, h->bspec, h->scratch, h->bufa, h->bufb})
+        if (p) cudaFree(p);
+    if (h->stream) cudaStreamDestroy(h->stream);
+    delete h;
+    return CB_OK;
+}
+
+int cb_fft_f64_size(const cb_fft_f64 *h, size_t *fft_size, int *inverse)
+{
+    CB_REQUIRE(h, CB_ERR_INVALID_ARG, "handle is NULL");
+    if (fft_size) *fft_size = h->n;
+    if (inverse) *inverse = h->inverse;
+    return CB_OK;
+}
+
+int cb_fft_f64_run_dev(cb_fft_f64 *h, const double *d_in, size_t n_in, double *d_out, void *stream)
+{
+    CB_REQUIRE(h, CB_ERR_INVALID_ARG, "handle is NULL");
+    CB_REQUIRE(n_in > 0 && n_in % h->n == 0, CB_ERR_SIZE, "fft_f64: input length %zu is not a multiple of fft_size %zu",
+               n_in, h->n);
+    CB_REQUIRE(d_in && d_out, CB_ERR_INVALID_ARG, "NULL data pointer");
+    CB_REQUIRE(((reinterpret_cast<uintptr_t>(d_in) | reinterpret_cast<uintptr_t>(d_out)) & 15) == 0, CB_ERR_INVALID_ARG,
+               "fft_f64: d_in and d_out must be 16-byte aligned");  // read and written as double2
+    CB_NO_ALIAS(d_in, n_in * sizeof(double2), d_out, n_in * sizeof(double2), "fft_f64");
+    CB_CUDA(cudaSetDevice(h->device));
+    cudaStream_t s = pick_stream(stream, h->stream);
+    int rc = h->last.begin(s);  // the two-step scratch and the chirp-z work buffers are per handle
+    if (rc) return rc;
+    rc = f64_exec(h, reinterpret_cast<const double2 *>(d_in), reinterpret_cast<double2 *>(d_out), n_in / h->n, s);
+    if (rc) return rc;
+    return h->last.end(s);
+}
+
+int cb_fft_f64_run(cb_fft_f64 *h, const double *in, size_t n_in, double *out)
+{
+    CB_REQUIRE(h, CB_ERR_INVALID_ARG, "handle is NULL");
+    CB_REQUIRE(n_in > 0 && n_in % h->n == 0, CB_ERR_SIZE, "fft_f64: input length %zu is not a multiple of fft_size %zu",
+               n_in, h->n);
+    CB_REQUIRE(in && out, CB_ERR_INVALID_ARG, "NULL data pointer");
+    CB_CUDA(cudaSetDevice(h->device));
+    const size_t N = h->n;
+    size_t chunk = HOST_CHUNK / N * N;
+    if (chunk == 0) chunk = N;
+    if (n_in < chunk) chunk = n_in;
+    int rc = h->last.sync();
+    if (rc) return rc;
+    rc = h->pipe.reserve(chunk * sizeof(double2), chunk * sizeof(double2));
+    if (rc) return rc;
+    rc = h->pipe.begin_call(in, n_in * sizeof(double2), chunk * sizeof(double2), out, n_in * sizeof(double2),
+                            chunk * sizeof(double2));
+    if (rc) return rc;
+    const double2 *hin = reinterpret_cast<const double2 *>(in);
+    double2 *hout = reinterpret_cast<double2 *>(out);
+    const bool shared = h->kind == F64_TWOSTEP || h->kind == F64_CHIRPZ;
+    size_t done = 0;
+    for (int i = 0; done < n_in; ++i) {
+        const int l = i & 1;
+        const size_t m = n_in - done < chunk ? n_in - done : chunk;
+        cudaStream_t s = h->pipe.lane[l];
+        double2 *di = reinterpret_cast<double2 *>(h->pipe.in[l]), *dout = reinterpret_cast<double2 *>(h->pipe.out[l]);
+        rc = h->pipe.h2d(l, di, hin + done, m * sizeof(double2));
+        if (rc) return rc;
+        if (shared && i > 0) CB_CUDA(cudaStreamSynchronize(h->pipe.lane[l ^ 1]));  // one scratch for both lanes
+        rc = f64_exec(h, di, dout, m / N, s);
+        if (rc) return rc;
+        rc = h->pipe.d2h(l, hout + done, dout, m * sizeof(double2));
         if (rc) return rc;
         done += m;
     }

@@ -347,6 +347,25 @@ struct FFTBatchNode : Node1<FFTBatchNode, std::vector<c32>, std::vector<c32>> {
     }
 };
 
+// FFTBatchNode<Complex<f64>>: the reference runs every transform in f64 (src/fft/mod.rs:73-96); see cb_fft_f64
+struct FFTBatchNodeF64 : Node1<FFTBatchNodeF64, std::vector<c64>, std::vector<c64>> {
+    cb_fft_f64 *h_ = nullptr;
+    FFTBatchNodeF64(size_t fft_size, bool ifft)
+    {
+        if (cb_fft_f64_create(fft_size, ifft, &h_)) throw std::runtime_error(cb_last_error());
+    }
+    ~FFTBatchNodeF64() { cb_fft_f64_destroy(h_); }
+    FFTBatchNodeF64(const FFTBatchNodeF64 &) = delete;
+    FFTBatchNodeF64 &operator=(const FFTBatchNodeF64 &) = delete;
+    Result<std::vector<c64>> run(const std::vector<c64> &in)
+    {
+        std::vector<c64> out(in.size());
+        int st = cb_fft_f64_run(h_, reinterpret_cast<const double *>(in.data()), in.size(),
+                                reinterpret_cast<double *>(out.data()));
+        return st ? Result<std::vector<c64>>::Err(map_status(st)) : Result<std::vector<c64>>::Ok(std::move(out));
+    }
+};
+
 // FFTSampleNode (#[aggregate]): emits only when fft_size samples have arrived   src/fft/fft_node.rs:101-168
 struct FFTSampleNode : Node1<FFTSampleNode, c32, std::vector<c32>, true> {
     cb_fft *h_ = nullptr;

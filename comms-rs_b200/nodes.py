@@ -435,6 +435,48 @@ class FFTSampleNode(FFTBatchNode):
         return None
 
 
+class FFTBatchNodeF64(_Handle):
+    """FFTBatchNode<Complex<f64>> (src/fft/fft_node.rs:65-74) over complex128: the transform the reference runs in f64
+    (src/fft/mod.rs:73-96), with the per-bin bound, determinism and edges stated in include/comms_b200.h (cb_fft_f64).
+    run() takes one frame or several contiguous frames."""
+
+    _destroy = "cb_fft_f64_destroy"
+
+    def __init__(self, fft_size: int, ifft: bool = False):
+        super().__init__()
+        self.fft_size = int(fft_size)
+        check(_lib.load().cb_fft_f64_create(self.fft_size, int(bool(ifft)), C.byref(self._h)))
+
+    def run(self, data) -> np.ndarray:
+        x = _c128(data).reshape(-1)
+        out = np.empty_like(x)
+        try:
+            check(_lib.load().cb_fft_f64_run(self._h, _ptr(x), len(x), _ptr(out)))
+        except CbError as e:
+            raise node_error(e) from e
+        return out
+
+    def run_dev(self, d_in: int, n_in: int, d_out: int, stream: int = 0) -> None:
+        """n_in complex f64 in and out; device pointers, 16-byte aligned."""
+        check(_lib.load().cb_fft_f64_run_dev(self._h, d_in, n_in, d_out, stream))
+
+
+class FFTSampleNodeF64(FFTBatchNodeF64):
+    """FFTSampleNode<Complex<f64>> (src/fft/fft_node.rs:101-168, #[aggregate]): collects samples; run() returns None
+    until fft_size samples have arrived."""
+
+    def __init__(self, fft_size: int, ifft: bool = False):
+        super().__init__(fft_size, ifft)
+        self._acc: list = []
+
+    def run(self, sample):  # type: ignore[override]
+        self._acc.append(sample)
+        if len(self._acc) == self.fft_size:
+            frame, self._acc = self._acc, []
+            return super().run(np.asarray(frame, dtype=np.complex128))
+        return None
+
+
 class FMDemodNode(_Handle):
     """FMDemodNode::new() (src/modulation/analog_node.rs:43-52)."""
 

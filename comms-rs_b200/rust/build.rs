@@ -24,7 +24,7 @@ fn main() {
         // the same list as comms-rs_b200/build.py (SOURCES)
         for f in ["api.cu", "comm.cu", "fir_kernels.cu", "fir_tc_kernel.cu", "fir_ptc_kernel.cu", "fir_real_kernel.cu", "fft_kernels.cu",
                   "fft_cluster_kernel.cu", "fft_cpipe_kernel.cu", "fft_rows_kernel.cu", "fft_big_kernel.cu", "chain_kernels.cu", "chain_tc_kernel.cu", "misc_kernels.cu",
-                  "estimator_kernels.cu", "nco_kernel.cu", "fir_f64_kernels.cu"] {
+                  "estimator_kernels.cu", "nco_kernel.cu", "fir_f64_kernels.cu", "fft_f64_kernels.cu"] {
             let p = csrc.join(f);
             println!("cargo:rerun-if-changed={}", p.display());
             cmd.arg(p);

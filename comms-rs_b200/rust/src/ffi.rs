@@ -3,7 +3,7 @@
 use std::os::raw::{c_char, c_double, c_float, c_int, c_uint, c_void};
 
 macro_rules! opaque { ($($n:ident),*) => { $(#[repr(C)] pub struct $n { _p: [u8; 0] })* } }
-opaque!(cb_stream, cb_buf, cb_fir, cb_mixer, cb_fft, cb_fm, cb_chain, cb_comm, cb_timing, cb_nco, cb_fir_f64);
+opaque!(cb_stream, cb_buf, cb_fir, cb_mixer, cb_fft, cb_fm, cb_chain, cb_comm, cb_timing, cb_nco, cb_fir_f64, cb_fft_f64);
 
 pub const CB_OK: c_int = 0;
 pub const CB_ERR_INVALID_ARG: c_int = 1;
@@ -85,6 +85,13 @@ extern "C" {
     pub fn cb_fft_run_dev(h: *mut cb_fft, d_in: *const c_float, n_in: usize, d_out: *mut c_float,
                           stream: *mut c_void) -> c_int;
     pub fn cb_fft_size(h: *const cb_fft, fft_size: *mut usize, inverse: *mut c_int) -> c_int;
+
+    pub fn cb_fft_f64_create(fft_size: usize, inverse: c_int, out: *mut *mut cb_fft_f64) -> c_int;
+    pub fn cb_fft_f64_destroy(h: *mut cb_fft_f64) -> c_int;
+    pub fn cb_fft_f64_size(h: *const cb_fft_f64, fft_size: *mut usize, inverse: *mut c_int) -> c_int;
+    pub fn cb_fft_f64_run(h: *mut cb_fft_f64, input: *const f64, n_in: usize, out: *mut f64) -> c_int;
+    pub fn cb_fft_f64_run_dev(h: *mut cb_fft_f64, d_in: *const f64, n_in: usize, d_out: *mut f64,
+                              stream: *mut c_void) -> c_int;
 
     pub fn cb_fm_create(out: *mut *mut cb_fm) -> c_int;
     pub fn cb_fm_destroy(h: *mut cb_fm) -> c_int;

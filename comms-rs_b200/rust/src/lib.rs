@@ -422,6 +422,69 @@ impl GpuFFTSampleNode {
     }
 }
 
+handle!(FftF64, ffi::cb_fft_f64, ffi::cb_fft_f64_destroy);
+
+fn fft_f64_new(fft_size: usize, ifft: bool) -> FftF64 {
+    let mut h = ptr::null_mut();
+    let st = unsafe { ffi::cb_fft_f64_create(fft_size, ifft as i32, &mut h) };
+    assert_eq!(st, ffi::CB_OK, "cb_fft_f64_create failed");
+    FftF64(h)
+}
+
+fn fft_f64_run(h: &FftF64, data: &[C64]) -> Result<Vec<C64>, NodeError> {
+    let mut out: Vec<C64> = Vec::with_capacity(data.len());
+    check(unsafe { ffi::cb_fft_f64_run(h.0, as_f64(data), data.len(), out.as_mut_ptr() as *mut f64) })?;
+    unsafe { out.set_len(data.len()) };
+    Ok(out)
+}
+
+/// Drop-in for `FFTBatchNode<f64>` (src/fft/fft_node.rs:26-84) over `Complex<f64>`: the reference runs every
+/// transform in f64 (src/fft/mod.rs:73-96), and so does `cb_fft_f64`.
+#[derive(Node)]
+#[pass_by_ref]
+pub struct GpuFFTBatchNodeF64 {
+    pub input: NodeReceiver<Vec<C64>>,
+    fft: FftF64,
+    pub output: NodeSender<Vec<C64>>,
+}
+
+impl GpuFFTBatchNodeF64 {
+    pub fn new(fft_size: usize, ifft: bool) -> Self {
+        GpuFFTBatchNodeF64 { fft: fft_f64_new(fft_size, ifft), input: Default::default(), output: Default::default() }
+    }
+    /// A length that is not a multiple of fft_size is a DataError (rustfft would panic the node thread).
+    pub fn run(&mut self, data: &[C64]) -> Result<Vec<C64>, NodeError> { fft_f64_run(&self.fft, data) }
+}
+
+/// Drop-in for `FFTSampleNode<f64>` (src/fft/fft_node.rs:101-168) over `Complex<f64>`.
+#[derive(Node)]
+#[aggregate]
+#[pass_by_ref]
+pub struct GpuFFTSampleNodeF64 {
+    pub input: NodeReceiver<C64>,
+    fft: FftF64,
+    fft_size: usize,
+    samples: Vec<C64>,
+    pub output: NodeSender<Vec<C64>>,
+}
+
+impl GpuFFTSampleNodeF64 {
+    pub fn new(fft_size: usize, ifft: bool) -> Self {
+        GpuFFTSampleNodeF64 { fft: fft_f64_new(fft_size, ifft), fft_size, samples: Vec::with_capacity(fft_size),
+                              input: Default::default(), output: Default::default() }
+    }
+    pub fn run(&mut self, input: &C64) -> Result<Option<Vec<C64>>, NodeError> {
+        self.samples.push(*input);
+        if self.samples.len() == self.fft_size {
+            let out = fft_f64_run(&self.fft, &self.samples)?;
+            self.samples.clear();
+            Ok(Some(out))
+        } else {
+            Ok(None)
+        }
+    }
+}
+
 /// Drop-in for `FMDemodNode<f32>` (src/modulation/analog_node.rs:18-52).
 #[derive(Node)]
 #[pass_by_ref]

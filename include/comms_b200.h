@@ -298,6 +298,55 @@ CB_API int cb_fft_size(const cb_fft *h, size_t *fft_size, int *inverse);
 CB_API int cb_fft_run_iq16(cb_fft *h, const int16_t *in, size_t n_in, float in_scale, float *out);
 CB_API int cb_fft_run_dev_iq16(cb_fft *h, const int16_t *d_in, size_t n_in, float in_scale, float *d_out, void *stream);
 
+/* ------------------------------------------------------------------ FFT over Complex<f64>
+ * BatchFFT::run_fft over Complex<f64> (src/fft/mod.rs:73-96 runs every transform in f64; FFTBatchNode<Complex<f64>>):
+ * cb_fft entry for entry (no i16 entries), with 2*n interleaved doubles wherever cb_fft has floats.  The same
+ * semantics: X[k] = sum_n x[n] exp(-/+ j 2 pi k n / N), "+" when inverse != 0, no 1/N in either direction; n_in a
+ * non-zero multiple of fft_size else CB_ERR_SIZE; the same overlap check; the per-handle scratch ordered across streams.
+ * d_in and d_out of cb_fft_f64_run_dev must be 16-byte aligned; other pointers return CB_ERR_INVALID_ARG before any
+ * launch.
+ * Limits.  Every power of two from 1 to 2^20 and every other length up to 2^19; anything larger returns
+ * CB_ERR_UNSUPPORTED from cb_fft_f64_create.  The plan picks its path from the size alone:
+ *   powers of two 8 .. 4096:      one CTA (or part of one) per frame, radix-8 Stockham passes in shared memory;
+ *   powers of two 8192 .. 2^20:   two steps N = N1 N2 (N1 = 2^floor(log2(N)/2)), the inter-step twiddle in between;
+ *   1, 2, 4 and other N <= 128:   direct sums over an exact-index table (kn mod N);
+ *   other N:                      chirp-z over M = the least power of two >= 2N - 1 (a power-of-two plan of M points).
+ * Numerical contract, per frame f of N points with u = 2^-53, S_f = sum_n |x[n]| and X the exact transform:
+ *   per bin:    |X'[k] - X[k]| <= tau * S_f + floor
+ *   per frame:  ||X' - X||_2 <= rho * ||X||_2 + sqrt(N) floor,     floor = 16 N 2^-1074 (chirp-z: 64 M sqrt(2N) 2^-1074)
+ *   powers of two (8 .. 4096):      tau = rho = 4 log2(N) u
+ *   powers of two (8192 .. 2^20):   tau = rho = (4 log2(N) + 4) u
+ *   direct sums (N <= 128):         tau = (3 N + 1) u,              rho = sqrt(N) tau
+ *   chirp-z:                        tau = sqrt(2N - 1) (8 log2(M) + 12) u + 8 u,   rho = sqrt(2) tau
+ * Derivation (first order in u; at log2 N <= 20 the second-order terms stay below 2^-40 of these).  Every
+ * intermediate of a power-of-two transform is a sum over a subset of the inputs times unit-modulus factors, and a
+ * rounding at one of them reaches each bin along one unit-modulus path; the subsets of one stage partition the frame,
+ * so a stage whose roundings are at most c u |v| adds c u S_f to every bin (and, in L2 norm, c u ||X||_2).  A complex
+ * addition rounds each part (u); the twiddle product re = fma(a.re, w.re, -(a.im w.im)), im = fma(a.re, w.im,
+ * a.im w.re) rounds twice per part (2 sqrt(2) u |a|), and the table entry, rounded once from long double, adds u |a|;
+ * the e^{-/+ i pi/4} products of the radix-8 butterfly round a sum, the constant and a product (3 u).  Per radix-8
+ * pass (three levels): twiddle 4 u + three additions 3 u + 3 u = 10 u < 4 u per level; a radix-4 pass 6 u, a radix-2
+ * pass 5 u (never alone: N >= 8).  The two-step form adds the inter-step twiddle (4 u).  A direct sum is two FMA
+ * chains of 2N terms per bin: gamma_2N on sum |x.re w.re| + |x.im w.im| <= S_f per part (2 sqrt(2) N u) plus the
+ * table (u); rho follows from ||e||_2 <= sqrt(N) max |e_k| and S_f <= ||X||_2.  Chirp-z: X[k] = w[k] c[k] with
+ * c = IFFT_M(FFT_M(x w) B / M), |c[k]| <= S_f; the pre- and post-products add 4 u each; an error e in the forward
+ * spectrum reaches c[k] as (1/M) sum_j e[j] B[j] e^{..}, at most tau_M S_f (1/M) sum_j |B[j]| <= tau_M S_f sqrt(2N - 1)
+ * (Cauchy-Schwarz, ||B||_2 = sqrt(M (2N - 1))), and likewise the inverse transform, the rounding of B / M (u) and the
+ * spectrum product (2 sqrt(2) u); with tau_M = (4 log2(M) + 4) u that is the tau above, and rho takes the trivial
+ * |B[j]| <= 2N - 1 in the L2 form.  The floor covers frames whose roundings fall in the subnormal range (2^-1075 per
+ * operation).
+ * Determinism.  A frame's output bits depend on its own samples and the plan alone: not on the batch size, the frame's
+ * position in the batch, how a stream of frames is split into calls, cb_fft_f64_run vs cb_fft_f64_run_dev, or the
+ * stream; they are bit-identical to the CPU emulation built from the same device code (tests/emul/fft_f64_emul.cpp).
+ * Edges.  A zero frame gives exact zeros.  An Inf or NaN makes every bin of its own frame non-finite and changes no
+ * other frame, including the other frames of a chirp-z or two-step group. */
+typedef struct cb_fft_f64 cb_fft_f64;
+CB_API int cb_fft_f64_create(size_t fft_size, int inverse, cb_fft_f64 **out);
+CB_API int cb_fft_f64_destroy(cb_fft_f64 *h);
+CB_API int cb_fft_f64_size(const cb_fft_f64 *h, size_t *fft_size, int *inverse);
+CB_API int cb_fft_f64_run(cb_fft_f64 *h, const double *in, size_t n_in, double *out);
+CB_API int cb_fft_f64_run_dev(cb_fft_f64 *h, const double *d_in, size_t n_in, double *d_out, void *stream);
+
 /* ------------------------------------------------------------------ FM demod
  * Replaces FM::demod (src/modulation/analog.rs:22-34): out[n] =
  * arg(x[n] * conj(x[n-1])), previous sample carried across calls, initially 0
